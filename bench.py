@@ -74,6 +74,11 @@ def parse_args():
                     help="CPU legs only: restrict the bounded sample to the first N stages (0 = all; used by the CPU unit test)")
     ap.add_argument("--profile", action="store_true",
                     help="for ncu: one warm-up replay + the timed steps only (no roofline graphs, no e2e, no CPU baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed seeded sample of every call's output of the last step (rank 0) "
+                         "as DIR/s<stage>_<site>.npy, float32 [depth, samples], to compare two builds output for output.  The output arena "
+                         "holds only the last 2 GiB of a step's output: every earlier call is launched once more, eagerly, on its "
+                         "input, so a defect that shows only under graph capture can be missing from those")
     return ap.parse_args()
 
 
@@ -266,6 +271,68 @@ class Arena:
         p = self.base + self.cur
         self.cur += nbytes_al
         return p
+
+
+def synthetic_step(torch, hot, dev, rank):
+    """The step's synthetic inputs, resident in HBM and the same on every run with the same workload and rank: the arenas,
+    the GALT factors and adaLN tensors of the rotate sites, and the plan, (call, input pointer, output pointer) per call."""
+    C = hot.width
+    g = torch.Generator(device=dev)
+    g.manual_seed(1234 + rank)
+    GiB = 1 << 30
+    a_f32 = torch.randn(GiB // 4 * 2, generator=g, device=dev, dtype=torch.float32)               # 2 GiB N(0,1) fp32
+    a_f16 = torch.randn(GiB // 2, generator=g, device=dev, dtype=torch.float32).to(torch.float16)  # 1 GiB N(0,1) fp16
+    a_gelu = torch.nn.functional.gelu(torch.randn(GiB, generator=g, device=dev, dtype=torch.float32), approximate="tanh").to(torch.float16)  # 2 GiB
+    a_out = torch.empty(2 * GiB, dtype=torch.uint8, device=dev)
+    arenas = {"f32": Arena(a_f32), "f16": Arena(a_f16), "gelu": Arena(a_gelu), "out": Arena(a_out)}
+    gs = torch.Generator(device="cpu"); gs.manual_seed(7)
+    smooth = {site: torch.exp(torch.rand(C, generator=gs) * 2 - 1).to(dev) for site in ("mat_qkv", "fc1")} if hot.rotate_transform else {}
+    modulate = {site: (1.0 + 0.3 * torch.randn(2 * hot.batch, C, generator=gs), 0.5 * torch.randn(2 * hot.batch, C, generator=gs))
+                for site in ("mat_qkv", "fc1")} if hot.modulate else {}
+    modulate = {k: (a.to(dev), b.to(dev)) for k, (a, b) in modulate.items()}
+    plan = [(c, in_arena(arenas, c).take(c.in_bytes), arenas["out"].take(c.out_bytes)) for c in hot.calls()]
+    return arenas, smooth, modulate, plan
+
+
+def in_arena(arenas, c):
+    """The input arena a call reads: fp32, GELU-skewed fp16 (fc2) or N(0,1) fp16."""
+    if c.in_dtype == "f32":
+        return arenas["f32"]
+    return arenas["gelu"] if c.site == "fc2" else arenas["f16"]
+
+
+DUMP_SAMPLES = 8192     # per call: the 1200 calls of the d30 step give 39 MB of float32
+
+
+def slice_intact(plan, i):
+    """Whether call i's output slice still holds its output at the end of the step: no later call of the plan writes into it."""
+    c, _, po = plan[i]
+    return all(q + d.out_bytes <= po or q >= po + c.out_bytes for d, _, q in plan[i + 1:])
+
+
+def dump_outputs(torch, np, path, plan, replay, out_arena, stream):
+    """--dump-outputs: a fixed sample (seeded by the call's index) of every call's output of the step just replayed, float32,
+    one [depth, samples] array per (stage, site).  The out arena is smaller than one step's output, so a later call of the
+    step may have written over an earlier call's slice: a slice left intact is sampled where the step wrote it, any other
+    call is launched once more on the same input into a scratch buffer (same kernel, same input bytes)."""
+    os.makedirs(path, exist_ok=True)
+    dev = out_arena.t.device
+    n = min(DUMP_SAMPLES, min(c.elems for c, _, _ in plan))
+    scratch = torch.empty(max(c.out_bytes for c, _, _ in plan), dtype=torch.uint8, device=dev)
+    rows = {}
+    torch.cuda.synchronize(dev)
+    with torch.cuda.stream(stream):
+        for i, (c, pi, po) in enumerate(plan):
+            if slice_intact(plan, i):
+                out = out_arena.t[po - out_arena.base:][:c.out_bytes]
+            else:
+                replay.launch(c, pi, scratch.data_ptr(), stream.cuda_stream)
+                out = scratch[:c.out_bytes]
+            idx = torch.from_numpy(np.random.default_rng(i).integers(0, c.elems, n)).to(dev)
+            vals = out.view(torch.float16 if c.out_dtype == "f16" else torch.float32)[idx].float()
+            rows.setdefault((c.stage, c.site), []).append(vals.cpu().numpy())
+    for (stage, site), r in rows.items():
+        np.save(os.path.join(path, f"s{stage}_{site}.npy"), np.stack(r))
 
 
 def config1_extra(torch, lib, dev, side):
@@ -570,30 +637,9 @@ def main():
     step_bytes = sum(c.bytes for c in calls)
     in_bytes = sum(c.in_bytes for c in calls)
     out_bytes = sum(c.out_bytes for c in calls)
-    C = hot.width
 
-    # ---- synthetic inputs, resident in HBM --------------------------------------------------
-    g = torch.Generator(device=dev)
-    g.manual_seed(1234 + rank)
-    GiB = 1 << 30
-    a_f32 = torch.randn(GiB // 4 * 2, generator=g, device=dev, dtype=torch.float32)               # 2 GiB N(0,1) fp32
-    a_f16 = torch.randn(GiB // 2, generator=g, device=dev, dtype=torch.float32).to(torch.float16)  # 1 GiB N(0,1) fp16
-    a_gelu = torch.nn.functional.gelu(torch.randn(GiB, generator=g, device=dev, dtype=torch.float32), approximate="tanh").to(torch.float16)  # 2 GiB
-    a_out = torch.empty(2 * GiB, dtype=torch.uint8, device=dev)
-    arenas = {"f32": Arena(a_f32), "f16": Arena(a_f16), "gelu": Arena(a_gelu), "out": Arena(a_out)}
-    gs = torch.Generator(device="cpu"); gs.manual_seed(7)
-    smooth = {site: torch.exp(torch.rand(C, generator=gs) * 2 - 1).to(dev) for site in ("mat_qkv", "fc1")} if hot.rotate_transform else {}
-    modulate = {site: (1.0 + 0.3 * torch.randn(2 * hot.batch, C, generator=gs), 0.5 * torch.randn(2 * hot.batch, C, generator=gs))
-                for site in ("mat_qkv", "fc1")} if hot.modulate else {}
-    modulate = {k: (a.to(dev), b.to(dev)) for k, (a, b) in modulate.items()}
+    arenas, smooth, modulate, plan = synthetic_step(torch, hot, dev, rank)
     replay = DeviceReplay(dev, smooth, modulate=modulate)
-
-    def in_arena(c):
-        if c.in_dtype == "f32":
-            return arenas["f32"]
-        return arenas["gelu"] if c.site == "fc2" else arenas["f16"]
-
-    plan = [(c, in_arena(c).take(c.in_bytes), arenas["out"].take(c.out_bytes)) for c in calls]
 
     def issue(subset, stream):
         for c, pi, po in subset:
@@ -636,6 +682,9 @@ def main():
     torch.cuda.synchronize()
     sampler = ClockSampler(local_rank) if rank == 0 else None
     t_dev = timed_replays(graph, args.steps)
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        dump_outputs(torch, np, args.dump_outputs, plan, replay, arenas["out"], side)
     if args.profile:
         if sampler:
             sampler.stop()
@@ -731,7 +780,7 @@ def main():
     # ---- the reference's own GPU path and its own model on this box (rank 0, N=1; outside every timed region above) ----
     reference_gpu = generation_ref = other = None
     if world == 1 and not args.no_reference_legs:
-        del replay, graph, big_graph, arenas, a_f32, a_f16, a_gelu, a_out, plan
+        del replay, graph, big_graph, arenas, plan
         torch.cuda.empty_cache()
         reference_gpu, generation_ref = reference_gpu_legs(torch, dev, hot, args)
     if world == 1 and not args.no_other_configs:

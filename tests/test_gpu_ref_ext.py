@@ -1,4 +1,4 @@
-"""GPU: the UNMODIFIED reference CUDA extension (compiled from /root/reference/quant into
+"""GPU: the UNMODIFIED reference CUDA extension (compiled from a checkout of the reference's quant/ sources into
 oracle/_ref by oracle/build_ref.sh) against (1) the oracle's restatement of its scan -- which
 closes the chain reference -> golden fixtures -- and (2) this repo's kernels, on the real device
 with real torch-CUDA glue arithmetic (fp16 division, type promotion)."""
@@ -17,7 +17,9 @@ pytestmark = pytest.mark.gpu
 def ref():
     mod = ref_glue.load_ref_ext()
     if mod is None:
-        pytest.skip("oracle/_ref/ref_quant_cuda*.so not built (needs /root/reference at build time)")
+        # no stored stand-in: these tests compare with the reference's own kernel, and without a build of it there is
+        # nothing of it to compare with (its outputs were never recorded)
+        pytest.skip("oracle/_ref/ref_quant_cuda*.so not built: oracle/build_ref.sh builds it from a checkout of the reference")
     return mod
 
 
