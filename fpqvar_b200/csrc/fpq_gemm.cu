@@ -11,10 +11,13 @@
 // At rest the FP4 formats shrink to 4 bits per element (fpq_codes_to_nibbles / fpq_nibbles_to_codes), same order.
 //
 // GEMM: C[m, n] = sum over slabs t of  sa[t, m] * sw[t, n] * P_t[m, n],   P_t = sum over the slab's 128 k of qa * qw,
-// P_t by tcgen05.mma kind::f8f6f4 (e4m3 x e4m3, fp32 accumulate in tensor memory; exact: every product is a multiple of 2^-8
-// and the sums stay far below 2^24 of them), the scale product by the epilogue warps on the CUDA cores while the tensor core
+// P_t by tcgen05.mma kind::f8f6f4 (e4m3 x e4m3, fp32 accumulate in tensor memory; exact while every partial sum fits fp32's 24
+// bits: k_acc * max|q_a| * max|q_w| / (u_a * u_w) <= 2^24, u the grid's resolution, k_acc = 128 with groups of 128 (every pair but
+// e3m2 x e3m2) and K with row scales (oracle/lowbit.py exact_accumulation); outside it P_t is within (k_acc - 1) * 2^-24 *
+// sum |qa * qw|), the scale product by the epilogue warps on the CUDA cores while the tensor core
 // works on the next slabs (512 columns of tensor memory: four 128-column or two 256-column accumulators).  The fp32 operation
-// order is fixed -- acc = fma(P*sa, sw, acc), slabs ascending -- so that oracle/gemm_codes.c reproduces C bit for bit.
+// order is fixed -- acc = fma(P*sa, sw, acc), slabs ascending -- so that oracle/gemm_codes.c reproduces C bit for bit inside the
+// envelope.
 //
 // Persistent kernel, one CTA per SM, 128 x 256 (or 128 x 128) tiles of C: warp 0 = bulk-copy producer, warp 1 = MMA issuer (one
 // lane), warps 4.. = epilogue (each owns 32 tensor-memory lanes -- its warp-id quarter -- and EC columns, read as 16 x 8

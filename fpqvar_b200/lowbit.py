@@ -3,8 +3,8 @@
 The reference's QuantizedLinear.forward is `act_quant(x)` -> `F.linear(q_x, W_q, b)` on fp16 tensors
 (models_fp_quant_transform_rotate/quant_utils.py:764-769).  Here the quantizer emits (grid value, scale per row and
 128-group) -- `PackedCodes` -- and `linear_codes` multiplies two of them on the tensor cores (csrc/fpq_gemm.cu, tcgen05.mma
-kind::f8f6f4).  `QuantizedLinearLowBit` is the module form: `from_quantized(QuantizedLinear)` packs the weight once, forward
-packs the activation and runs the GEMM.  No fallback: without the CUDA library every call raises.
+kind::f8f6f4).  `QuantizedLinearLowBit` is the module form: `from_float(nn.Linear)` packs the weight once, forward packs the
+activation and runs the GEMM.  No fallback: without the CUDA library every call raises.
 """
 from __future__ import annotations
 
@@ -158,16 +158,25 @@ def linear_codes_sse(a: PackedCodes, w: PackedCodes, ref: torch.Tensor, bias: Op
     m, n = a.rows, w.rows
     if a.k != w.k or (a.scale_group == GROUP) != (w.scale_group == GROUP):
         raise L.FpqError("linear_codes_sse: operands do not match")
-    if ref.dtype not in _DT or ref.shape != (m, n) or not ref.is_contiguous() or n % 8 != 0:
-        raise L.FpqError("linear_codes_sse: ref must be a contiguous float16 / float32 [m, n] tensor, n a multiple of 8")
+    if a.codes.device != w.codes.device:
+        raise L.FpqError("linear_codes_sse: operands on different devices")
+    if ref.dtype not in _DT or ref.shape != (m, n) or not ref.is_contiguous() or n % 8 != 0 or ref.device != a.codes.device:
+        raise L.FpqError("linear_codes_sse: ref must be a contiguous float16 / float32 [m, n] tensor on the operands' device, "
+                         "n a multiple of 8")
     if sse is None:
         sse = torch.zeros(1, dtype=torch.float64, device=ref.device)
-    elif sse.dtype != torch.float64 or not sse.is_cuda or sse.numel() < 1:
-        raise L.FpqError("linear_codes_sse: sse must be a float64 CUDA tensor")
-    b = None if bias is None else bias.detach().to(torch.float32).contiguous()
+    elif sse.dtype != torch.float64 or not sse.is_cuda or sse.numel() < 1 or sse.device != a.codes.device:
+        raise L.FpqError("linear_codes_sse: sse must be a float64 CUDA tensor on the operands' device")
+    b = None
+    if bias is not None:
+        _require_cuda(bias, "linear_codes_sse(bias)")
+        if bias.numel() != n:
+            raise L.FpqError(f"linear_codes_sse: bias has {bias.numel()} entries, expected {n}")
+        b = bias.detach().to(device=a.codes.device, dtype=torch.float32).contiguous()
     if row_weight is not None and (row_weight.dtype != torch.float64 or not row_weight.is_cuda or row_weight.numel() != m
-                                   or not row_weight.is_contiguous()):
-        raise L.FpqError("linear_codes_sse: row_weight must be a contiguous float64 CUDA tensor with one entry per row")
+                                   or not row_weight.is_contiguous() or row_weight.device != a.codes.device):
+        raise L.FpqError("linear_codes_sse: row_weight must be a contiguous float64 tensor on the operands' device with one "
+                         "entry per row")
     with _on_device(a.codes) as dev:
         L.check(L.lib().fpq_gemm_codes_sse(a.codes.data_ptr(), a.scales.data_ptr(), m, w.codes.data_ptr(), w.scales.data_ptr(), n, a.k,
                                            a.scale_group, None if b is None else b.data_ptr(), _DT[ref.dtype], ref.data_ptr(), n,

@@ -261,7 +261,12 @@ FPQ_API int fpq_selftest_f16_flow(int format, unsigned long long *result, void *
  * (row, 128-group) -- and the product runs on the tensor cores in 8-bit containers (tcgen05.mma kind::f8f6f4), the scales
  * applied per 128-deep K slab.  Numerics contract: fpq_unpack_codes(fpq_pack_codes(x)) is bit-identical to
  * fp_quant_*_per_group_cuda(x) (qu.py:265-378, :537-574; the reference's dtype rules: an fp16 input has an fp16-rounded scale);
- * fpq_gemm_codes is bit-identical to oracle/gemm_codes.c (fixed fp32 operation order) and differs from the reference's fp16
+ * fpq_gemm_codes is bit-identical to oracle/gemm_codes.c (fixed fp32 operation order) inside the exact-accumulation envelope
+ *   k_acc * max|q_a| * max|q_w| / (u_a * u_w) <= 2^24        (u: the grid's resolution; k_acc = 128 with groups of 128, k with
+ *                                                              row scales; oracle/lowbit.py exact_accumulation)
+ * where every partial sum of a scale group is an fp32 number: every 128-group pair but e3m2 x e3m2 (24.6 bits); with row scales
+ * e3m0 x e3m0 up to k = 4096, e2m1 x e2m1 up to k = 116480, FP6 pairs far less (e3m2 x e3m2 not even at k = 2304).  Outside
+ * it a slab sum may differ from the exact one by (k_acc - 1) * 2^-24 * sum |qa * qw|.  It differs from the reference's fp16
  * GEMM of the fake-quantized tensors only by that GEMM's own roundings (each product term fp16-rounded once in the reference,
  * never here; tolerance stated in tests/test_gpu_gemm_codes.py).
  *
@@ -289,8 +294,9 @@ FPQ_API int fpq_nibbles_to_codes(const uint8_t *nibbles, size_t n_codes, int for
 /*
  * F.linear(A, W, bias) for A = [m, k] and W = [n, k] given as codes that share `scale_group` (128 or k):
  *   C[i, j] = bias[j] + fma-chain over the scale groups t (ascending) of  (P_t[i, j] * sa[t, i]) * sw[t, j],
- *             P_t[i, j] = sum over the group's k of qa[i, k] * qw[j, k]        (fp32 accumulate in tensor memory; exact for the
- *                                                                              FP4 formats and for 128-groups of the FP6 ones)
+ *             P_t[i, j] = sum over the group's k of qa[i, k] * qw[j, k]        (fp32 accumulate in tensor memory; exact inside
+ *                                                                              the envelope above, within (k_acc - 1) * 2^-24 *
+ *                                                                              sum |qa * qw| outside it)
  * c: [m, ldc] row-major, FPQ_F16 | FPQ_F32, 16-byte aligned, n % 8 == 0, ldc % 8 == 0; bias: fp32 [n] or NULL.
  * Persistent kernel, one CTA per SM, 128 x 256 (or 128 x 128) tiles of C, ~205 KB of shared memory.  With groups of 128 every
  * accumulator is handed to the epilogue warps once per 128 K (1.0-1.45 PFLOP/s on a B200); with row scales once per tile

@@ -5,8 +5,12 @@
  * QuantizedLinear.forward (models_fp_quant_transform_rotate/quant_utils.py:764-769) for operands given as
  * (grid value, scale per row and 128-group) pairs instead of the fp16 tensors q * scale the reference materialises
  * (qu.py:313-330).  Operation order of the fp32 arithmetic, which the CUDA kernel follows to the letter:
- *     for group t = 0 .. K/group - 1: P = sum_{k in group} qa[i,k] * qw[j,k]    (exact: small dyadic rationals; the tensor core
- *                                    accumulates in fp32, which is exact too while |P| * 2^8 < 2^24: always for the FP4 formats)
+ *     for group t = 0 .. K/group - 1: P = sum_{k in group} qa[i,k] * qw[j,k]    (exact here, in double; the tensor core
+ *                                    accumulates in fp32, which is exact too while every partial sum fits 24 bits:
+ *                                    group * max|qa| * max|qw| / (u_a * u_w) <= 2^24, u the grid's resolution
+ *                                    (oracle/lowbit.py exact_accumulation: every 128-group pair but e3m2 x e3m2; one scale
+ *                                    per row: e3m0 x e3m0 up to K = 4096).  Outside it the kernel's P may differ from this
+ *                                    one by (group - 1) * 2^-24 * sum |qa * qw|)
  *                                    acc = fmaf( P * sa[t,i]  (rounded to fp32),  sw[t,j],  acc )
  *     c[i,j] = acc + bias[j]
  * "parity unpinned" by the reference (it has no such operator); pinned instead against a float64 evaluation of the

@@ -135,8 +135,9 @@ def test_gemm_codes_many_tiles_per_cta():
                                                ("e3m2", "e3m2", np.float16)])
 def test_row_scaled_codes_and_gemm(fmt_a, fmt_w, dtype):
     """per_token activations x per_channel weights (the README's W6A6 commands; fp6_quant_*_per_token_cuda qu.py:503-534):
-    one scale per row, the whole K accumulates in tensor memory.  FP4: bit-exact (the sums are exact in fp32); FP6: the
-    accumulation order inside the tensor core is not specified, tolerance 2^-20 of sum |terms|."""
+    one scale per row, the whole K accumulates in tensor memory.  Inside the exact-accumulation envelope (LB.exact_accumulation:
+    every partial sum is an fp32 number) bit-exact; outside it the fp32 sums may round: tolerance 2^-20 of sum |terms| (the
+    contract's bound is (K - 1) * 2^-24; on these normal-distributed operands the rounding errors stay far below it)."""
     rng = np.random.default_rng(13)
     m, n, k = 300, 384, 2304
     x = rng.standard_normal((m, k)).astype(dtype)
@@ -151,7 +152,7 @@ def test_row_scaled_codes_and_gemm(fmt_a, fmt_w, dtype):
     (qa, sa), (qw, sw) = LB.quantize_codes(x, fmt_a, None), LB.quantize_codes(w, fmt_w, None)
     c = lowbit.linear_codes(a, ww, None, torch.float32).cpu().numpy()
     want = LB.gemm_codes(qa, sa, qw, sw)
-    if fmt_a in ("e2m1", "e1m2", "e3m0"):
+    if LB.exact_accumulation(fmt_a, fmt_w, k):
         assert np.array_equal(bits(c), bits(want))
     else:
         mag = (np.abs(qa) * sa) @ (np.abs(qw) * sw).T
