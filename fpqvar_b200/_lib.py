@@ -40,6 +40,11 @@ SIGNATURES = {
     "fpq_modulate_transform_rotate_quant": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p,
                                                        _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_size_t, _c.c_int, _c.c_int,
                                                        _c.c_void_p]),
+    "fpq_transform_rotate_pack_codes": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t,
+                                                   _c.c_size_t, _c.c_int, _c.c_void_p]),
+    "fpq_modulate_transform_rotate_pack_codes": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p,
+                                                            _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_size_t, _c.c_int,
+                                                            _c.c_int, _c.c_void_p]),
     "fpq_transform_rotate_weight": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_size_t,
                                                _c.c_void_p]),
     "fpq_score_formats": (_c.c_int, [_c.c_void_p, _c.c_size_t, _c.c_size_t, _c.c_int, _c.c_void_p, _c.c_int, _c.c_int,

@@ -32,10 +32,8 @@
 //   groups of 128 1.04-1.49 PFLOP/s: the epilogue's 2 flops per element (512 clk of the fp32 pipe per 128 x 256 slab, as long as
 //   the slab's MMAs) and its tensor-memory loads do not fully overlap with a memory-bound main loop; DESIGN.md 3.6 has the
 //   experiments (tcgen05.ld alone: ~1 KB/clk per SM, tools/tmem_ldbench.cu; epilogue compiled out; per-tile overhead).
-#include "fpq_common.cuh"
+#include "fpq_codes.cuh"
 #include "fpq_stream.cuh"
-#include <cuda_fp8.h>
-#include <type_traits>
 
 namespace fpq {
 
@@ -49,65 +47,8 @@ constexpr uint32_t A_BYTES = TM * GK, SA_BYTES = TM * 4;
 // ---------------------------------------------------------------------------------------------------------------------
 // quantizer -> codes.  One warp per (8 rows x 128 K) block: lane = (row & 7) + 8 * (chunk & 3), two chunks of 16 elements per
 // lane, so that a warp reads 8 x 128 contiguous bytes (fp16) per instruction pair and writes 512 contiguous bytes per store.
-// Arithmetic: the reference's own sequence (qu.py:313-330 and Appendix A of SURVEY.md); see grid_values16.
+// Arithmetic: the reference's own sequence (qu.py:313-330 and Appendix A of SURVEY.md); see grid_values16 (fpq_codes.cuh).
 // ---------------------------------------------------------------------------------------------------------------------
-template <typename T> struct Chunk16;
-template <> struct Chunk16<__half> {
-    static __device__ __forceinline__ void load(const __half* p, float (&v)[16]) {
-        const uint4 a = ldg_stream(p), b = ldg_stream(p + 8);
-        const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            v[2 * i] = h2f(uint16_t(w[i] & 0xffffu));
-            v[2 * i + 1] = h2f(uint16_t(w[i] >> 16));
-        }
-    }
-    static __device__ __forceinline__ float scale(float amax, float vmax) { return __half2float(__float2half_rn(__fdiv_rn(amax, vmax))); }
-    static __device__ __forceinline__ float norm(float x, float s) { return __half2float(__float2half_rn(__fdiv_rn(x, s))); }
-};
-template <> struct Chunk16<float> {
-    static __device__ __forceinline__ void load(const float* p, float (&v)[16]) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const uint4 a = ldg_stream(p + 4 * j);
-            v[4 * j] = __uint_as_float(a.x); v[4 * j + 1] = __uint_as_float(a.y);
-            v[4 * j + 2] = __uint_as_float(a.z); v[4 * j + 3] = __uint_as_float(a.w);
-        }
-    }
-    static __device__ __forceinline__ float scale(float amax, float vmax) { return __fdiv_rn(amax, vmax); }
-    static __device__ __forceinline__ float norm(float x, float s) { return __fdiv_rn(x, s); }
-};
-
-__device__ __forceinline__ uint32_t e4m3x4(float a, float b, float c, float d) {
-    const uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(a, b), __NV_SATFINITE, __NV_E4M3);
-    const uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(c, d), __NV_SATFINITE, __NV_E4M3);
-    return lo | (hi << 16);
-}
-
-// Grid values of 16 elements that share the scale s.  fp16 tensors with a regular scale (normal, finite: everything but zero,
-// tiny, inf and NaN groups) take the division-free element function of the packed fp16 quantizers (fpq_h16.cuh: half(x * RN(1/s))
-// == half(x / s), tie shift 2^-17, magic-number rounding; checked against the literal sequence for every (x, scale) pair by
-// fpq_selftest_f16_flow) -- the grid value is that function's intermediate; everything else takes the literal sequence.
-template <typename T, class HG>
-__device__ __forceinline__ void grid_values16(const float (&v)[16], float s, float delta, float (&q)[16]) {
-    if constexpr (std::is_same<T, __half>::value) {
-        if (scale_bits_regular(uint32_t(__half_as_ushort(__float2half_rn(s))))) {
-            const float r = rcp_rn_normal(s);
-            const uint64_t r2 = pk(r, r);
-#pragma unroll
-            for (int i = 0; i < 16; i += 2) {
-                const uint32_t v2 = pack_h2_u64(fmul2(pk(v[i], v[i + 1]), r2));                      // half(x/s)
-                const F2 f = unpk(round_pair_magic(fhadd(uint16_t(v2 & 0xffffu), delta), fhadd(uint16_t(v2 >> 16), delta), Magic<HG>::EM, Magic<HG>::SC));
-                q[i] = f.lo;
-                q[i + 1] = f.hi;
-            }
-            return;
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < 16; ++i) q[i] = round_any_sym<HG, TIE_KERNEL>(Chunk16<T>::norm(v[i], s));
-}
-
 template <typename T, class HG>
 __global__ void __launch_bounds__(256) pack_codes_kernel(const T* __restrict__ x, size_t rows, size_t rows_pad, size_t k,
                                                          uint8_t* __restrict__ codes, float* __restrict__ scales) {

@@ -5,6 +5,8 @@
 // Q = I (x) diag(sigma) H_128 / fl32(sqrt(128)) (rotation_utils.py:69-104, hadamard_utils.py:63-99),
 // so (x @ Q) on an aligned 128-chunk is FWHT_128(x * sigma) / c: 7 butterfly stages instead of a
 // dense C x C GEMM.
+// Both activation kernels write either fp16 (fake-quantized, or rotated only) or, with CODES, the packed operand of the low-bit
+// GEMM (fpq_*transform_rotate_pack_codes: e4m3 grid value per element + scale per (row, 128-chunk), fpq_gemm.cu's layout).
 //
 // Numerics shared by the two activation kernels below (so that a row rotates to the same bits whichever
 // kernel the launcher picks for the tensor's size; test_rotation_bits_do_not_depend_on_the_launch_size):
@@ -13,6 +15,7 @@
 //   * a Sylvester Hadamard transform is the tensor product of a 2-point butterfly (a + b, a - b) over every
 //     index bit of the chunk position, in any order; the order fixes the fp32 summation tree and is
 //     0, 1, 5, 6, 2, 3, 4 in both kernels.
+#include "fpq_codes.cuh"
 #include "fpq_stream.cuh"
 
 namespace fpq {
@@ -21,6 +24,54 @@ struct SignMask { uint32_t w[4]; };    // bit e of the 128-bit mask set  <=>  si
 
 // adaLN modulate operands (fpq_modulate_transform_rotate_quant): t = (x * (scale[b, c] + 1) + shift[b, c]) * smooth[c]
 struct Modulate { const float* scale; const float* shift; size_t rows_per_batch; float one; };   // one: 1.0f, or -0.0f (the exact additive identity) under FPQ_MOD_GAIN
+
+// Codes output (fpq_*transform_rotate_pack_codes): the layout of include/fpq_b200.h, rows_pad = fpq_codes_rows_padded(n_rows).
+// The kernels that write it store, per element, the grid value the fp16 output would have multiplied by the group's scale, and
+// per (row, 128-chunk) that scale: the bytes fpq_pack_codes writes for the fp16 rotated tensor.
+struct CodesOut { uint8_t* codes; float* scales; size_t rows_pad; };
+constexpr uint32_t CODES_BLOCK_BYTES = 1024;          // 8 rows x 128 K: one row block of a slab
+
+// Codes output: the padding rows n_rows .. rows_pad - 1 of every slab get code 0 and scale 0 from the same launch, spread over
+// all of its threads (fewer than 128 rows per slab: one 16-byte store per thread or less at the sizes of a VAR pass).
+__device__ __forceinline__ void zero_codes_padding(const CodesOut& co, size_t n_rows, int cpr) {
+    const size_t pad = co.rows_pad - n_rows;
+    const size_t per_slab = pad * 9;                   // eight 16-byte code pieces and one scale per padding row
+    const size_t total = per_slab * size_t(cpr);
+    for (size_t u = size_t(blockIdx.x) * blockDim.x + threadIdx.x; u < total; u += size_t(gridDim.x) * blockDim.x) {
+        const size_t slab = u / per_slab, v = u % per_slab;
+        if (v < pad * 8) {
+            const size_t row = n_rows + v / 8;
+            *reinterpret_cast<uint4*>(co.codes + (slab * (co.rows_pad / 8) + row / 8) * CODES_BLOCK_BYTES + (v & 7) * 128 + (row & 7) * 16) =
+                make_uint4(0u, 0u, 0u, 0u);
+        } else {
+            co.scales[slab * co.rows_pad + n_rows + (v - pad * 8)] = 0.0f;
+        }
+    }
+}
+
+// Codes of 16 fp16 values of a group with an irregular scale (the literal sequence, out of line).  The values go through a
+// copy, so that the caller's register tile itself never needs an address.
+template <class HG>
+__device__ __forceinline__ uint4 irregular_codes16(const uint32_t* w, float s, float delta) {
+    uint32_t t[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) t[i] = w[i];
+    return codes16_h16<HG>(t, s, delta);
+}
+// The same for a streaming lane's 32 values, stored as its two K pieces (dst, dst + 128) by the out-of-line function itself,
+// so that nothing of the caller's but the loop state is live across the call.
+template <class HG>
+static __device__ __noinline__ void codes32_store_h16(const uint32_t* w, float s, float delta, uint8_t* dst) {
+    stg_stream(dst, codes16_h16<HG>(w, s, delta));
+    stg_stream(dst + 128, codes16_h16<HG>(w + 8, s, delta));
+}
+template <class HG>
+__device__ __forceinline__ void irregular_codes32(const uint32_t* w, float s, float delta, uint8_t* dst) {
+    uint32_t t[16];
+#pragma unroll
+    for (int i = 0; i < 16; ++i) t[i] = w[i];
+    codes32_store_h16<HG>(t, s, delta, dst);
+}
 
 // 1 / fl32(sqrt(128)), rounded to fp32 (SURVEY.md section 7: 0x3DB504F3)
 __device__ __forceinline__ float inv_sqrt128() { return __uint_as_float(0x3DB504F3u); }
@@ -91,11 +142,13 @@ __device__ __forceinline__ void pair_stage(uint64_t (&P)[N]) {
 // fp32, sm_100): P[2j] = (v[4j], v[4j+1]), P[2j+1] = (v[4j+2], v[4j+3]).
 // MOD (adaLN modulate fused in): a lane set walks CONTIGUOUS rows (k0*R .. k0*R + R - 1) instead of strided ones, so
 // the (scale+1) and shift values of its column change only when the batch index does and live in registers in between.
+// CODES (codes output instead of `out` / `rotated`): lane l's four 4-element pieces are 4-byte pieces of codes, 256 B apart.
 // ------------------------------------------------------------------------------------------------------------
-template <int FMT, bool QUANT, bool MOD>
+template <int FMT, bool QUANT, bool MOD, bool CODES>
 __global__ void __launch_bounds__(256, MOD ? 1 : 0) transform_rotate_quant_small_kernel(const float* __restrict__ x, const float* __restrict__ smooth,
                                                                                        SignMask sm, __half* __restrict__ out, __half* __restrict__ rotated,
-                                                                                       size_t n_rows, int cpr, size_t sets_per_col, Modulate mod) {
+                                                                                       size_t n_rows, int cpr, size_t sets_per_col, Modulate mod,
+                                                                                       CodesOut co) {
     constexpr int LPG = 8;
     pdl_launch_dependents();
     const int lane = threadIdx.x & 31;
@@ -164,6 +217,22 @@ __global__ void __launch_bounds__(256, MOD ? 1 : 0) transform_rotate_quant_small
         uint32_t w[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) w[i] = pack_h2_u64(P[i]);
+        if constexpr (CODES) {
+            float s;
+            const bool ok = sym_quant_tile_h16<FMT, LPG, 8, true, true>(w, s, delta);
+            if (valid) {
+                const uint4 c = ok ? make_uint4(e4m3x4_h2(w[0], w[1]), e4m3x4_h2(w[2], w[3]), e4m3x4_h2(w[4], w[5]), e4m3x4_h2(w[6], w[7]))
+                                   : irregular_codes16<typename SymFmt<FMT>::HG>(w, s, delta);
+                // element 32 j + 4 lig + k: K piece 2 j + lig / 4, byte 4 (lig % 4) + k
+                uint8_t* cb = co.codes + (size_t(cc) * (co.rows_pad / 8) + row / 8) * CODES_BLOCK_BYTES + (row & 7) * 16 + (lig >> 2) * 128 + (lig & 3) * 4;
+                *reinterpret_cast<uint32_t*>(cb) = c.x;
+                *reinterpret_cast<uint32_t*>(cb + 256) = c.y;
+                *reinterpret_cast<uint32_t*>(cb + 512) = c.z;
+                *reinterpret_cast<uint32_t*>(cb + 768) = c.w;
+                if (lig == 0) co.scales[size_t(cc) * co.rows_pad + row] = s;
+            }
+            continue;
+        }
         if (valid && rotated != nullptr) {
 #pragma unroll
             for (int j = 0; j < 4; ++j) stg_stream(rotated + off + (j * LPG + lig) * 4, make_uint2(w[2 * j], w[2 * j + 1]));
@@ -179,6 +248,7 @@ __global__ void __launch_bounds__(256, MOD ? 1 : 0) transform_rotate_quant_small
             if (!ok) literal_sym_h16(out + off, out + off, lig, LPG, 4, 4, s, SymFmt<FMT>::GT);
         }
     }
+    if constexpr (CODES) zero_codes_padding(co, n_rows, cpr);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -219,7 +289,9 @@ constexpr int ROT_WARP_SMEM = 2 * ROT_WARP_STAGE_BYTES + 16;      // + the two m
 // element on 64-bit row arithmetic, re-derived shared-memory addresses and branches): rows are 32-bit counters relative to
 // the CTA's first row, global pointers are advanced instead of recomputed, every shared-memory address is a lane constant
 // plus an immediate, and the two buffers are two copies of the step body with compile-time offsets.
-template <int FMT, bool QUANT, bool MOD>
+// CODES: pass 2's 32 contiguous elements of a lane are two 16-byte K pieces of codes of one row, 128 B apart (an 8-row line is
+// completed over four steps of the same warp and merged in L2); the padding rows are written at the end of the launch.
+template <int FMT, bool QUANT, bool MOD, bool CODES>
 struct RotStream {
     // lane constants
     uint32_t p1;            // pass 1: this lane's first unit of its chunk (row 0, buffer 0)
@@ -239,6 +311,10 @@ struct RotStream {
     // output
     __half* op;             // this lane's 32 output elements of row `row2` of the current step
     __half* rp;             // same in `rotated` (or nullptr)
+    // CODES output: two 32-bit counters only (the addresses are rebuilt from the kernel parameters every step; 64-bit pointers
+    // here pushed the plain kernel past its 96 registers)
+    uint32_t cslab;         // this lane's chunk column (slab)
+    uint32_t crow;          // row `row2` of the current step (the launcher keeps rows_pad below 2^32)
 
     // this lane's (scale + 1) and shift of the batch `pa` / `psh` point at
     __device__ __forceinline__ void load_operands() {
@@ -306,7 +382,7 @@ struct RotStream {
             Q[2 * i + 1] = (uint64_t(u.w) << 32) | u.z;
         }
     }
-    __device__ __forceinline__ void pass2_finish(bool valid, uint64_t (&Q)[16]) {
+    __device__ __forceinline__ void pass2_finish(bool valid, uint64_t (&Q)[16], const CodesOut& co) {
         reg_stage(Q, 2);                // index bit 2
         reg_stage(Q, 4);                // index bit 3
         reg_stage(Q, 8);                // index bit 4
@@ -314,6 +390,22 @@ struct RotStream {
         uint32_t w[16];
 #pragma unroll
         for (int i = 0; i < 16; ++i) w[i] = pack_h2_u64(Q[i]);
+        if constexpr (CODES) {
+            float sc;
+            const bool ok = sym_quant_tile_h16<FMT, 4, 16, ROT_HW_QUANT, true>(w, sc, delta);
+            if (valid) {
+                uint8_t* p = co.codes + (size_t(cslab) * (co.rows_pad / 8) + (crow >> 3)) * CODES_BLOCK_BYTES + uint32_t(lq) * 256u + (crow & 7u) * 16u;
+                if (ok) {
+                    stg_stream(p, make_uint4(e4m3x4_h2(w[0], w[1]), e4m3x4_h2(w[2], w[3]), e4m3x4_h2(w[4], w[5]), e4m3x4_h2(w[6], w[7])));
+                    stg_stream(p + 128, make_uint4(e4m3x4_h2(w[8], w[9]), e4m3x4_h2(w[10], w[11]), e4m3x4_h2(w[12], w[13]), e4m3x4_h2(w[14], w[15])));
+                } else {
+                    irregular_codes32<typename SymFmt<FMT>::HG>(w, sc, delta, p);
+                }
+                if (lq == 0) co.scales[size_t(cslab) * co.rows_pad + crow] = sc;
+            }
+            crow += 2;
+            return;
+        }
         if (rp != nullptr) {
             if (valid) {
 #pragma unroll
@@ -335,10 +427,10 @@ struct RotStream {
     }
 };
 
-template <int FMT, bool QUANT, bool MOD>
+template <int FMT, bool QUANT, bool MOD, bool CODES>
 __device__ __forceinline__ void rotate_stream_body(const float* __restrict__ x, const float* __restrict__ smooth,
                                                    SignMask sm, __half* __restrict__ out, __half* __restrict__ rotated,
-                                                   size_t n_rows, int cpr, Modulate mod) {
+                                                   size_t n_rows, int cpr, Modulate mod, const CodesOut& co) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_warps = blockDim.x >> 5;
@@ -361,7 +453,7 @@ __device__ __forceinline__ void rotate_stream_body(const float* __restrict__ x, 
     const int col0 = 4 * warp;                                          // first chunk column of this warp
     const int ncols = cpr - col0 < 4 ? cpr - col0 : 4;                  // its columns that exist (the last warp may own fewer)
 
-    RotStream<FMT, QUANT, MOD> st;
+    RotStream<FMT, QUANT, MOD, CODES> st;
     const uint32_t smem_base = smem_u32(stage0);
     // pass 1: 8 lanes per chunk; sub-iteration = row, g4 = column within the warp
     const int g4 = lane >> 3, l8 = lane & 7;
@@ -387,6 +479,10 @@ __device__ __forceinline__ void rotate_stream_body(const float* __restrict__ x, 
     st.mod_one = mod.one;
     st.op = out + (r_begin + size_t(st.row2)) * row_elems + size_t(col0 + c2) * 128 + st.lq * 32;
     st.rp = rotated != nullptr ? rotated + (r_begin + size_t(st.row2)) * row_elems + size_t(col0 + c2) * 128 + st.lq * 32 : nullptr;
+    if constexpr (CODES) {
+        st.cslab = uint32_t(col0 + c2);
+        st.crow = uint32_t(r_begin) + uint32_t(st.row2);
+    }
     st.pa = st.psh = nullptr;
     st.left = st.rpb = 1;
     st.reload = false;
@@ -448,7 +544,7 @@ __device__ __forceinline__ void rotate_stream_body(const float* __restrict__ x, 
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
         issue(s);                       // step k + 2 into the buffer step k just left
-        st.pass2_finish(valid, Q);
+        st.pass2_finish(valid, Q, co);
     };
     uint32_t phase = 0;
     for (uint32_t done = 0; done < n_mine; done += 4u) {
@@ -456,21 +552,22 @@ __device__ __forceinline__ void rotate_stream_body(const float* __restrict__ x, 
         if (done + 2u < n_mine) step(1, done + 2u, phase);
         phase ^= 1u;
     }
+    if constexpr (CODES) zero_codes_padding(co, n_rows, cpr);
 }
 
 // Registers: about 20 resident warps per SM at 96 registers; the adaLN variant keeps 32 more operands live and gets 128
 // (16 warps).
-template <int FMT, bool QUANT>
+template <int FMT, bool QUANT, bool CODES>
 __global__ void __maxnreg__(96) transform_rotate_quant_stream_kernel(const float* __restrict__ x, const float* __restrict__ smooth,
                                                                     SignMask sm, __half* __restrict__ out, __half* __restrict__ rotated,
-                                                                    size_t n_rows, int cpr, Modulate mod) {
-    rotate_stream_body<FMT, QUANT, false>(x, smooth, sm, out, rotated, n_rows, cpr, mod);
+                                                                    size_t n_rows, int cpr, Modulate mod, CodesOut co) {
+    rotate_stream_body<FMT, QUANT, false, CODES>(x, smooth, sm, out, rotated, n_rows, cpr, mod, co);
 }
-template <int FMT, bool QUANT>
+template <int FMT, bool QUANT, bool CODES>
 __global__ void __maxnreg__(128) modulate_transform_rotate_quant_stream_kernel(const float* __restrict__ x, const float* __restrict__ smooth,
                                                                               SignMask sm, __half* __restrict__ out, __half* __restrict__ rotated,
-                                                                              size_t n_rows, int cpr, Modulate mod) {
-    rotate_stream_body<FMT, QUANT, true>(x, smooth, sm, out, rotated, n_rows, cpr, mod);
+                                                                              size_t n_rows, int cpr, Modulate mod, CodesOut co) {
+    rotate_stream_body<FMT, QUANT, true, CODES>(x, smooth, sm, out, rotated, n_rows, cpr, mod, co);
 }
 
 // Weight side: one warp per (row, chunk); lane l holds elements 4l..4l+3 in fp64.  w_out may alias w (in place): every
@@ -535,12 +632,12 @@ static bool rot_plan(int cpr, bool mod, RotPlan& p) {
     return true;
 }
 
-template <int FMT, bool QUANT, bool MOD>
-static int launch_stream(const float* x, const float* smooth, const SignMask& sm, __half* o, __half* rot, size_t n_rows, int cpr,
-                         const RotPlan& plan, const Modulate& m, cudaStream_t st) {
-    void (*kernel)(const float*, const float*, SignMask, __half*, __half*, size_t, int, Modulate);
-    if constexpr (MOD) kernel = modulate_transform_rotate_quant_stream_kernel<FMT, QUANT>;
-    else kernel = transform_rotate_quant_stream_kernel<FMT, QUANT>;
+template <int FMT, bool QUANT, bool MOD, bool CODES>
+static int launch_stream(const float* x, const float* smooth, const SignMask& sm, __half* o, __half* rot, const CodesOut& co, size_t n_rows,
+                         int cpr, const RotPlan& plan, const Modulate& m, cudaStream_t st) {
+    void (*kernel)(const float*, const float*, SignMask, __half*, __half*, size_t, int, Modulate, CodesOut);
+    if constexpr (MOD) kernel = modulate_transform_rotate_quant_stream_kernel<FMT, QUANT, CODES>;
+    else kernel = transform_rotate_quant_stream_kernel<FMT, QUANT, CODES>;
     const size_t smem = size_t(plan.warps) * ROT_WARP_SMEM;
     static bool attr_done[64] = {};                    // per instantiation and device
     int dev = 0;
@@ -552,13 +649,13 @@ static int launch_stream(const float* x, const float* smooth, const SignMask& sm
     const size_t steps = (n_rows + 1) / 2;
     const size_t cap = size_t(sm_count()) * plan.ctas_per_sm;
     const unsigned grid = unsigned(steps < cap ? steps : cap);
-    launch_pdl(kernel, grid, unsigned(32 * plan.warps), smem, st, x, smooth, sm, o, rot, n_rows, cpr, m);
+    launch_pdl(kernel, grid, unsigned(32 * plan.warps), smem, st, x, smooth, sm, o, rot, n_rows, cpr, m, co);
     return finish_launch();
 }
 
-template <int FMT, bool QUANT, bool MOD>
-static int launch_small(const float* x, const float* smooth, const SignMask& sm, __half* o, __half* rot, size_t n_rows, int cpr,
-                        const Modulate& m, cudaStream_t st) {
+template <int FMT, bool QUANT, bool MOD, bool CODES>
+static int launch_small(const float* x, const float* smooth, const SignMask& sm, __half* o, __half* rot, const CodesOut& co, size_t n_rows,
+                        int cpr, const Modulate& m, cudaStream_t st) {
     // lane sets, one per (chunk column, row phase); enough to fill every SM's thread slots (the modulate variant holds
     // three operand tables in registers: 2 resident CTAs instead of 4)
     const size_t max_sets = size_t(sm_count()) * (MOD ? 1024 : 2048) / 8;
@@ -570,48 +667,74 @@ static int launch_small(const float* x, const float* smooth, const SignMask& sm,
     sets_per_col = (n_rows + trips - 1) / trips;
     const size_t n_sets = sets_per_col * size_t(cpr);
     const unsigned grid = unsigned((n_sets + 31) / 32);            // 32 lane sets per 256-thread block
-    launch_pdl(transform_rotate_quant_small_kernel<FMT, QUANT, MOD>, grid, 256, 0, st, x, smooth, sm, o, rot, n_rows, cpr, sets_per_col, m);
+    launch_pdl(transform_rotate_quant_small_kernel<FMT, QUANT, MOD, CODES>, grid, 256, 0, st, x, smooth, sm, o, rot, n_rows, cpr, sets_per_col, m, co);
     return finish_launch();
 }
 
-template <int FMT, bool QUANT>
-static int launch_fmt(const float* x, const Modulate* mod, const float* smooth, const SignMask& sm, __half* o, __half* rot, size_t n_rows, int cpr,
-                      cudaStream_t st) {
+template <int FMT, bool QUANT, bool CODES>
+static int launch_fmt(const float* x, const Modulate* mod, const float* smooth, const SignMask& sm, __half* o, __half* rot, const CodesOut& co,
+                      size_t n_rows, int cpr, cudaStream_t st) {
     const Modulate m = mod ? *mod : Modulate{nullptr, nullptr, 1, 1.0f};
     RotPlan plan;
     const bool big = n_rows * size_t(cpr) > size_t(g_tun.rot_small_max_chunks) && rot_plan(cpr, mod != nullptr, plan) &&
                      (mod == nullptr || mod->rows_per_batch >= 2) &&
                      ((reinterpret_cast<uintptr_t>(o) | reinterpret_cast<uintptr_t>(rot)) & 15) == 0;      // 128-bit stores
-    if (big) return mod ? launch_stream<FMT, QUANT, true>(x, smooth, sm, o, rot, n_rows, cpr, plan, m, st) : launch_stream<FMT, QUANT, false>(x, smooth, sm, o, rot, n_rows, cpr, plan, m, st);
-    return mod ? launch_small<FMT, QUANT, true>(x, smooth, sm, o, rot, n_rows, cpr, m, st) : launch_small<FMT, QUANT, false>(x, smooth, sm, o, rot, n_rows, cpr, m, st);
+    if (big) return mod ? launch_stream<FMT, QUANT, true, CODES>(x, smooth, sm, o, rot, co, n_rows, cpr, plan, m, st)
+                        : launch_stream<FMT, QUANT, false, CODES>(x, smooth, sm, o, rot, co, n_rows, cpr, plan, m, st);
+    return mod ? launch_small<FMT, QUANT, true, CODES>(x, smooth, sm, o, rot, co, n_rows, cpr, m, st)
+               : launch_small<FMT, QUANT, false, CODES>(x, smooth, sm, o, rot, co, n_rows, cpr, m, st);
 }
 
-static int launch_rotate_quant(const float* x, const Modulate* mod, const float* smooth, const uint32_t* sign_bits_host, void* out, void* rotated,
-                               size_t n_rows, size_t n_cols, int format, void* stream) {
-    if (n_cols == 0 || n_cols % 128 != 0 || n_cols / 128 > 0x7fffffff / 512 || !sign_bits_host || (n_rows && (!x || !out))) return FPQ_ERR_ARG;
-    if (format < -1 || format >= FPQ_NUM_SYM_FORMATS) return FPQ_ERR_ARG;
-    if (((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(smooth)) & 15) || (reinterpret_cast<uintptr_t>(out) & 7) ||
-        (reinterpret_cast<uintptr_t>(rotated) & 7))
-        return FPQ_ERR_ARG;
+// Checks shared by both outputs
+static int check_rotate_args(const float* x, const Modulate* mod, const float* smooth, const uint32_t* sign_bits_host, size_t n_rows, size_t n_cols) {
+    if (n_cols == 0 || n_cols % 128 != 0 || n_cols / 128 > 0x7fffffff / 512 || !sign_bits_host || (n_rows && !x)) return FPQ_ERR_ARG;
+    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(smooth)) & 15) return FPQ_ERR_ARG;
     if (mod != nullptr) {
         if (!mod->scale || !mod->shift || mod->rows_per_batch == 0 || n_rows % mod->rows_per_batch != 0) return FPQ_ERR_ARG;
         if ((reinterpret_cast<uintptr_t>(mod->scale) | reinterpret_cast<uintptr_t>(mod->shift)) & 15) return FPQ_ERR_ARG;
     }
-    if (n_rows == 0) return FPQ_OK;
+    return FPQ_OK;
+}
+
+// format: FPQ_FMT_*, or -1 (rotation only) for the fp16 output
+template <bool CODES>
+static int launch_rotate(const float* x, const Modulate* mod, const float* smooth, const uint32_t* sign_bits_host, __half* o, __half* rot,
+                         const CodesOut& co, size_t n_rows, size_t n_cols, int format, void* stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     SignMask sm;
     for (int i = 0; i < 4; ++i) sm.w[i] = sign_bits_host[i];
     const int cpr = int(n_cols / 128);
-    __half* o = static_cast<__half*>(out);
-    __half* rot = static_cast<__half*>(rotated);
     switch (format) {
-        case -1: return launch_fmt<0, false>(x, mod, smooth, sm, o, rot, n_rows, cpr, st);
-        case FPQ_FMT_E2M1: return launch_fmt<FPQ_FMT_E2M1, true>(x, mod, smooth, sm, o, rot, n_rows, cpr, st);
-        case FPQ_FMT_E1M2: return launch_fmt<FPQ_FMT_E1M2, true>(x, mod, smooth, sm, o, rot, n_rows, cpr, st);
-        case FPQ_FMT_E3M0: return launch_fmt<FPQ_FMT_E3M0, true>(x, mod, smooth, sm, o, rot, n_rows, cpr, st);
-        case FPQ_FMT_E2M3: return launch_fmt<FPQ_FMT_E2M3, true>(x, mod, smooth, sm, o, rot, n_rows, cpr, st);
-        default: return launch_fmt<FPQ_FMT_E3M2, true>(x, mod, smooth, sm, o, rot, n_rows, cpr, st);
+        case FPQ_FMT_E2M1: return launch_fmt<FPQ_FMT_E2M1, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
+        case FPQ_FMT_E1M2: return launch_fmt<FPQ_FMT_E1M2, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
+        case FPQ_FMT_E3M0: return launch_fmt<FPQ_FMT_E3M0, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
+        case FPQ_FMT_E2M3: return launch_fmt<FPQ_FMT_E2M3, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
+        case FPQ_FMT_E3M2: return launch_fmt<FPQ_FMT_E3M2, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
+        default: break;
     }
+    if constexpr (!CODES) return launch_fmt<0, false, false>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
+    return FPQ_ERR_ARG;
+}
+
+static int launch_rotate_quant(const float* x, const Modulate* mod, const float* smooth, const uint32_t* sign_bits_host, void* out, void* rotated,
+                               size_t n_rows, size_t n_cols, int format, void* stream) {
+    if (int rc = check_rotate_args(x, mod, smooth, sign_bits_host, n_rows, n_cols)) return rc;
+    if ((n_rows && !out) || format < -1 || format >= FPQ_NUM_SYM_FORMATS) return FPQ_ERR_ARG;
+    if ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(rotated)) & 7) return FPQ_ERR_ARG;
+    if (n_rows == 0) return FPQ_OK;
+    return launch_rotate<false>(x, mod, smooth, sign_bits_host, static_cast<__half*>(out), static_cast<__half*>(rotated), CodesOut{nullptr, nullptr, 0},
+                                n_rows, n_cols, format, stream);
+}
+
+static int launch_rotate_codes(const float* x, const Modulate* mod, const float* smooth, const uint32_t* sign_bits_host, uint8_t* codes, float* scales,
+                               size_t n_rows, size_t n_cols, int format, void* stream) {
+    if (int rc = check_rotate_args(x, mod, smooth, sign_bits_host, n_rows, n_cols)) return rc;
+    if ((n_rows && (!codes || !scales)) || format < 0 || format >= FPQ_NUM_SYM_FORMATS) return FPQ_ERR_ARG;
+    if ((reinterpret_cast<uintptr_t>(codes) & 15) || (reinterpret_cast<uintptr_t>(scales) & 3)) return FPQ_ERR_ARG;
+    if (n_rows == 0) return FPQ_OK;
+    if (fpq_codes_rows_padded(n_rows) > 0xFFFFFFFFull) return FPQ_ERR_UNSUPPORTED;      // the streaming kernel counts rows in 32 bits
+    return launch_rotate<true>(x, mod, smooth, sign_bits_host, nullptr, nullptr, CodesOut{codes, scales, fpq_codes_rows_padded(n_rows)}, n_rows,
+                               n_cols, format, stream);
 }
 
 // Introspection for the CPU tests (tests/rotate_layout_model.py mirrors the launcher): plan[2] = {warps per CTA, CTAs per SM}.
@@ -635,6 +758,19 @@ extern "C" int fpq_modulate_transform_rotate_quant(const float* x, const float* 
     if (flags & ~FPQ_MOD_GAIN) return FPQ_ERR_ARG;
     const Modulate m{scale, shift, rows_per_batch, (flags & FPQ_MOD_GAIN) ? -0.0f : 1.0f};
     return launch_rotate_quant(x, &m, smooth, sign_bits_host, out, rotated, n_rows, n_cols, format, stream);
+}
+
+extern "C" int fpq_transform_rotate_pack_codes(const float* x, const float* smooth, const uint32_t* sign_bits_host, uint8_t* codes, float* scales,
+                                               size_t n_rows, size_t n_cols, int format, void* stream) {
+    return launch_rotate_codes(x, nullptr, smooth, sign_bits_host, codes, scales, n_rows, n_cols, format, stream);
+}
+
+extern "C" int fpq_modulate_transform_rotate_pack_codes(const float* x, const float* scale, const float* shift, size_t rows_per_batch,
+                                                        const float* smooth, const uint32_t* sign_bits_host, uint8_t* codes, float* scales,
+                                                        size_t n_rows, size_t n_cols, int format, int flags, void* stream) {
+    if (flags & ~FPQ_MOD_GAIN) return FPQ_ERR_ARG;
+    const Modulate m{scale, shift, rows_per_batch, (flags & FPQ_MOD_GAIN) ? -0.0f : 1.0f};
+    return launch_rotate_codes(x, &m, smooth, sign_bits_host, codes, scales, n_rows, n_cols, format, stream);
 }
 
 extern "C" int fpq_transform_rotate_weight(const float* w, const float* smooth, const uint32_t* sign_bits_host, float* w_out, size_t n_rows,

@@ -103,20 +103,63 @@ const float* smooth_ptr(c10::optional<at::Tensor>& smooth, const at::Tensor& x, 
     return s.data_ptr<float>();
 }
 
+// Arguments of the rotate operators, checked and converted in one place for both outputs (fp16 and codes).  `scale` / `shift`
+// present: the adaLN-modulated entry, x = [B, ..., C] with [B, 1, C] operands.  The device guard lives as long as the call.
+struct RotateCall {
+    c10::cuda::OptionalCUDAGuard guard;
+    at::Tensor x;
+    at::Tensor mods[2];                 // fp32 gain or scale, fp32 shift (modulated entry only)
+    const float* sp = nullptr;          // smooth
+    uint32_t bits[4] = {0, 0, 0, 0};
+    size_t rows = 0, cols = 0, rows_per_batch = 0;
+    int flags = 0;
+
+    RotateCall(at::Tensor x_, const at::Tensor* scale, const at::Tensor* shift, c10::optional<at::Tensor>& smooth, const std::vector<int64_t>& sign_bits,
+               const std::string& what) {
+        const bool mod = scale != nullptr;
+        require_cuda(x_, what.c_str());
+        if (!mod && x_.scalar_type() != at::kFloat) throw std::runtime_error(what + ": x must be float32 (the adaLN-modulated LayerNorm output)");
+        if (mod && (x_.scalar_type() != at::kFloat || x_.dim() < 2)) throw std::runtime_error(what + ": x must be float32 [B, ..., C]");
+        if (sign_bits.size() != 4) throw std::runtime_error(what + ": sign_bits must hold 4 words");
+        guard.set_device(x_.device());
+        x = x_.contiguous();
+        const int64_t c = x.dim() > 0 ? x.size(-1) : 0;
+        cols = size_t(c);
+        rows = c ? size_t(x.numel() / c) : 0;
+        if (mod) {
+            const int64_t b = x.size(0);
+            const int64_t rpb = (b * c) ? x.numel() / (b * c) : 0;
+            mods[0] = scale->detach();
+            mods[1] = shift->detach();
+            const char* names[2] = {"scale", "shift"};
+            for (int i = 0; i < 2; ++i) {
+                const at::Tensor& t = mods[i];
+                require_cuda(t, (what + "(scale/shift)").c_str());
+                if (t.numel() != b * c || t.dim() < 1 || t.size(0) != b || t.size(-1) != c)
+                    throw std::runtime_error(std::string(names[i]) + " must be [B, 1, C] = [" + std::to_string(b) + ", 1, " + std::to_string(c) + "]");
+                if (t.scalar_type() != at::kFloat && t.scalar_type() != at::kHalf) throw std::runtime_error(std::string(names[i]) + " must be float32 or float16");
+            }
+            // fp16 adaLN tensors (the reference's fp16 autocast): `scale.add(1)` is an fp16 add there; do it with the same ATen op on
+            // the tiny [B, 1, C] tensor and hand the rounded result to the kernel as a gain
+            if (mods[0].scalar_type() == at::kHalf) { mods[0] = mods[0].add(1); flags = FPQ_MOD_GAIN; }
+            for (auto& t : mods) t = t.to(at::kFloat).contiguous();
+            rows_per_batch = size_t(rpb);
+            rows = size_t(b * rpb);
+        }
+        sp = smooth_ptr(smooth, x, c, (what + "(smooth)").c_str());
+        for (int i = 0; i < 4; ++i) bits[i] = uint32_t(sign_bits[i]);
+    }
+    const float* scale_ptr() const { return mods[0].data_ptr<float>(); }
+    const float* shift_ptr() const { return mods[1].data_ptr<float>(); }
+};
+
 std::vector<at::Tensor> transform_rotate_quant(at::Tensor x, c10::optional<at::Tensor> smooth, std::vector<int64_t> sign_bits, int64_t format, bool want_rotated) {
-    require_cuda(x, "transform_rotate_quant");
-    if (x.scalar_type() != at::kFloat) throw std::runtime_error("transform_rotate_quant: x must be float32 (the adaLN-modulated LayerNorm output)");
-    if (sign_bits.size() != 4) throw std::runtime_error("transform_rotate_quant: sign_bits must hold 4 words");
-    c10::cuda::CUDAGuard guard(x.device());
-    x = x.contiguous();
-    const int64_t c = x.dim() > 0 ? x.size(-1) : 0;
-    const float* sp = smooth_ptr(smooth, x, c, "transform_rotate_quant(smooth)");
-    at::Tensor out = at::empty(x.sizes(), x.options().dtype(at::kHalf));
+    RotateCall r(x, nullptr, nullptr, smooth, sign_bits, "transform_rotate_quant");
+    at::Tensor out = at::empty(r.x.sizes(), r.x.options().dtype(at::kHalf));
     at::Tensor rot;
     if (want_rotated) rot = at::empty_like(out);
-    const uint32_t bits[4] = {uint32_t(sign_bits[0]), uint32_t(sign_bits[1]), uint32_t(sign_bits[2]), uint32_t(sign_bits[3])};
-    check_rc(fpq_transform_rotate_quant(x.data_ptr<float>(), sp, bits, out.data_ptr(), want_rotated ? rot.data_ptr() : nullptr,
-                                        c ? size_t(x.numel() / c) : 0, size_t(c), int(format), stream_of(x)),
+    check_rc(fpq_transform_rotate_quant(r.x.data_ptr<float>(), r.sp, r.bits, out.data_ptr(), want_rotated ? rot.data_ptr() : nullptr, r.rows, r.cols,
+                                        int(format), stream_of(r.x)),
              "fpq_transform_rotate_quant");
     if (want_rotated) return {out, rot};
     return {out};
@@ -124,38 +167,43 @@ std::vector<at::Tensor> transform_rotate_quant(at::Tensor x, c10::optional<at::T
 
 std::vector<at::Tensor> modulate_transform_rotate_quant(at::Tensor x, at::Tensor scale, at::Tensor shift, c10::optional<at::Tensor> smooth,
                                                         std::vector<int64_t> sign_bits, int64_t format, bool want_rotated) {
-    require_cuda(x, "modulate_transform_rotate_quant");
-    if (x.scalar_type() != at::kFloat || x.dim() < 2) throw std::runtime_error("modulate_transform_rotate_quant: x must be float32 [B, ..., C]");
-    if (sign_bits.size() != 4) throw std::runtime_error("modulate_transform_rotate_quant: sign_bits must hold 4 words");
-    c10::cuda::CUDAGuard guard(x.device());
-    x = x.contiguous();
-    const int64_t b = x.size(0), c = x.size(-1);
-    const int64_t rpb = (b * c) ? x.numel() / (b * c) : 0;
-    int flags = 0;
-    at::Tensor mods[2] = {scale.detach(), shift.detach()};
-    const char* names[2] = {"scale", "shift"};
-    for (int i = 0; i < 2; ++i) {
-        const at::Tensor& t = mods[i];
-        require_cuda(t, "modulate_transform_rotate_quant(scale/shift)");
-        if (t.numel() != b * c || t.dim() < 1 || t.size(0) != b || t.size(-1) != c)
-            throw std::runtime_error(std::string(names[i]) + " must be [B, 1, C] = [" + std::to_string(b) + ", 1, " + std::to_string(c) + "]");
-        if (t.scalar_type() != at::kFloat && t.scalar_type() != at::kHalf) throw std::runtime_error(std::string(names[i]) + " must be float32 or float16");
-    }
-    // fp16 adaLN tensors (the reference's fp16 autocast): `scale.add(1)` is an fp16 add there; do it with the same ATen op on
-    // the tiny [B, 1, C] tensor and hand the rounded result to the kernel as a gain
-    if (mods[0].scalar_type() == at::kHalf) { mods[0] = mods[0].add(1); flags = FPQ_MOD_GAIN; }
-    for (auto& t : mods) t = t.to(at::kFloat).contiguous();
-    const float* sp = smooth_ptr(smooth, x, c, "modulate_transform_rotate_quant(smooth)");
-    at::Tensor out = at::empty(x.sizes(), x.options().dtype(at::kHalf));
+    RotateCall r(x, &scale, &shift, smooth, sign_bits, "modulate_transform_rotate_quant");
+    at::Tensor out = at::empty(r.x.sizes(), r.x.options().dtype(at::kHalf));
     at::Tensor rot;
     if (want_rotated) rot = at::empty_like(out);
-    const uint32_t bits[4] = {uint32_t(sign_bits[0]), uint32_t(sign_bits[1]), uint32_t(sign_bits[2]), uint32_t(sign_bits[3])};
-    check_rc(fpq_modulate_transform_rotate_quant(x.data_ptr<float>(), mods[0].data_ptr<float>(), mods[1].data_ptr<float>(), size_t(rpb), sp, bits,
-                                                 out.data_ptr(), want_rotated ? rot.data_ptr() : nullptr, size_t(b * rpb), size_t(c), int(format), flags,
-                                                 stream_of(x)),
+    check_rc(fpq_modulate_transform_rotate_quant(r.x.data_ptr<float>(), r.scale_ptr(), r.shift_ptr(), r.rows_per_batch, r.sp, r.bits, out.data_ptr(),
+                                                 want_rotated ? rot.data_ptr() : nullptr, r.rows, r.cols, int(format), r.flags, stream_of(r.x)),
              "fpq_modulate_transform_rotate_quant");
     if (want_rotated) return {out, rot};
     return {out};
+}
+
+// codes output: (codes uint8 [rows_pad * C], scales fp32 [C / 128, rows_pad]), the operand layout of fpq_gemm_codes
+std::vector<at::Tensor> codes_buffers(const RotateCall& r) {
+    const size_t rows_pad = fpq_codes_rows_padded(r.rows);
+    at::Tensor codes = at::empty({int64_t(rows_pad * r.cols)}, r.x.options().dtype(at::kByte));
+    at::Tensor scales = at::empty({int64_t(r.cols / 128), int64_t(rows_pad)}, r.x.options().dtype(at::kFloat));
+    return {codes, scales};
+}
+
+std::vector<at::Tensor> transform_rotate_pack_codes(at::Tensor x, c10::optional<at::Tensor> smooth, std::vector<int64_t> sign_bits, int64_t format) {
+    RotateCall r(x, nullptr, nullptr, smooth, sign_bits, "transform_rotate_pack_codes");
+    std::vector<at::Tensor> o = codes_buffers(r);
+    check_rc(fpq_transform_rotate_pack_codes(r.x.data_ptr<float>(), r.sp, r.bits, o[0].data_ptr<uint8_t>(), o[1].data_ptr<float>(), r.rows, r.cols,
+                                             int(format), stream_of(r.x)),
+             "fpq_transform_rotate_pack_codes");
+    return o;
+}
+
+std::vector<at::Tensor> modulate_transform_rotate_pack_codes(at::Tensor x, at::Tensor scale, at::Tensor shift, c10::optional<at::Tensor> smooth,
+                                                             std::vector<int64_t> sign_bits, int64_t format) {
+    RotateCall r(x, &scale, &shift, smooth, sign_bits, "modulate_transform_rotate_pack_codes");
+    std::vector<at::Tensor> o = codes_buffers(r);
+    check_rc(fpq_modulate_transform_rotate_pack_codes(r.x.data_ptr<float>(), r.scale_ptr(), r.shift_ptr(), r.rows_per_batch, r.sp, r.bits,
+                                                      o[0].data_ptr<uint8_t>(), o[1].data_ptr<float>(), r.rows, r.cols, int(format), r.flags,
+                                                      stream_of(r.x)),
+             "fpq_modulate_transform_rotate_pack_codes");
+    return o;
 }
 
 }  // namespace
@@ -167,6 +215,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.def("fake_quant_signsplit", &fake_quant_signsplit);
     m.def("transform_rotate_quant", &transform_rotate_quant);
     m.def("modulate_transform_rotate_quant", &modulate_transform_rotate_quant);
+    m.def("transform_rotate_pack_codes", &transform_rotate_pack_codes);
+    m.def("modulate_transform_rotate_pack_codes", &modulate_transform_rotate_pack_codes);
     m.def("launch_count", []() { return fpq_launch_count(); });
     m.def("version", []() { return std::string(fpq_version()); });
 }

@@ -4,7 +4,9 @@ The reference's QuantizedLinear.forward is `act_quant(x)` -> `F.linear(q_x, W_q,
 (models_fp_quant_transform_rotate/quant_utils.py:764-769).  Here the quantizer emits (grid value, scale per row and
 128-group) -- `PackedCodes` -- and `linear_codes` multiplies two of them on the tensor cores (csrc/fpq_gemm.cu, tcgen05.mma
 kind::f8f6f4).  `QuantizedLinearLowBit` is the module form: `from_float(nn.Linear)` packs the weight once, forward packs the
-activation and runs the GEMM.  No fallback: without the CUDA library every call raises.
+activation and runs the GEMM.  `rotate_pack_codes` emits the codes of a rotated / transformed linear's input (mat_qkv, fc1)
+straight out of the fused rotate kernel, for `QuantizedLinearLowBit.forward_packed`.  No fallback: without the CUDA library
+every call raises.
 """
 from __future__ import annotations
 
@@ -14,7 +16,7 @@ from typing import Optional
 import torch
 
 from . import _lib as L
-from .ops import _on_device, _require_cuda, _stream
+from .ops import _call, _ext, _on_device, _require_cuda, _stream
 
 _DT = {torch.float32: L.FPQ_F32, torch.float16: L.FPQ_F16}
 GROUP = 128
@@ -112,6 +114,33 @@ def pack_codes(x: torch.Tensor, fmt: str, per_row: bool = False) -> PackedCodes:
         L.check(L.lib().fpq_pack_codes(x2.data_ptr(), rows, k, sg, _DT[x2.dtype], L.FMT[fmt], codes.data_ptr(), scales.data_ptr(),
                                        _stream(dev)), f"fpq_pack_codes({fmt})")
     return PackedCodes(codes, scales, rows, k, fmt, sg)
+
+
+def rotate_pack_codes(x: torch.Tensor, smooth: Optional[torch.Tensor], sign_bits, fmt: str, scale: Optional[torch.Tensor] = None,
+                      shift: Optional[torch.Tensor] = None) -> PackedCodes:
+    """ops.transform_rotate_quant (scale / shift given: ops.modulate_transform_rotate_quant) with the quantized activation
+    emitted as codes, scales per (row, 128-group), in one launch (fpq_transform_rotate_pack_codes): bit-identical to
+    pack_codes(<the same call with fmt=None>, fmt).  x: fp32 [..., C] ([B, ..., C] with [B, 1, C] scale / shift),
+    C % 128 == 0; rows = x.numel() // C."""
+    _require_cuda(x, "rotate_pack_codes")
+    if fmt is None or fmt not in L.FMT:
+        raise L.FpqError(f"rotate_pack_codes: a quantizer format is required (one of {sorted(L.FMT)}); got {fmt!r}")
+    if (scale is None) != (shift is None):
+        raise L.FpqError("rotate_pack_codes: scale and shift go together")
+    if x.dtype != torch.float32 or x.dim() < (2 if scale is not None else 1):
+        raise L.FpqError("rotate_pack_codes: x must be a float32 tensor" + (" [B, ..., C]" if scale is not None else " [..., C]"))
+    c = x.shape[-1]
+    if c == 0 or c % GROUP != 0:
+        raise L.FpqError(f"rotate_pack_codes: last dim {c} is not a positive multiple of {GROUP}")
+    for t, name in ((scale, "scale"), (shift, "shift"), (smooth, "smooth")):
+        if t is not None:
+            _require_cuda(t, f"rotate_pack_codes({name})")
+    bits = list(sign_bits)
+    if scale is None:
+        codes, scales = _call(_ext().transform_rotate_pack_codes, x, smooth, bits, L.FMT[fmt])
+    else:
+        codes, scales = _call(_ext().modulate_transform_rotate_pack_codes, x, scale, shift, smooth, bits, L.FMT[fmt])
+    return PackedCodes(codes, scales, x.numel() // c, c, fmt, GROUP)
 
 
 def linear_codes(a: PackedCodes, w: PackedCodes, bias: Optional[torch.Tensor] = None, out_dtype=torch.float16,
@@ -217,6 +246,16 @@ class QuantizedLinearLowBit(torch.nn.Module):
         a = pack_codes(x, self.act_fmt, self.per_row)
         y = linear_codes(a, self.weight_packed(), self.bias, self.out_dtype)
         return y.reshape(*x.shape[:-1], self.out_features)
+
+    def forward_packed(self, a: PackedCodes) -> torch.Tensor:
+        """The product of an activation that is already packed (rotate_pack_codes): [a.rows, out_features].  `a` must carry
+        this module's activation format and scale grouping."""
+        if a.fmt != self.act_fmt:
+            raise L.FpqError(f"forward_packed: activation codes are {a.fmt}, this layer quantizes activations as {self.act_fmt}")
+        if (a.scale_group != GROUP) != self.per_row:
+            raise L.FpqError("forward_packed: activation scales are " + ("per row" if a.scale_group != GROUP else "per 128-group")
+                             + ", this layer expects " + ("per row" if self.per_row else "per 128-group"))
+        return linear_codes(a, self.weight_packed(), self.bias, self.out_dtype)
 
     def extra_repr(self) -> str:
         return (f"{self.in_features}, {self.out_features}, bias={self.bias is not None}, weight={self.weight_fmt} codes, "

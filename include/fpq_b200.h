@@ -27,6 +27,7 @@
  *   fpq_score_formats         search/search_fp4_format.py:340-374,472-476,840-893 and
  *                             search/search_fp6_format.py:547-554 (tensor-level quantize + MSE)
  *   fpq_pack_codes / fpq_gemm_codes   QuantizedLinear.forward qu.py:764-769 (act_quant + F.linear) as a real low-bit GEMM
+ *   fpq_[modulate_]transform_rotate_pack_codes   basic_var.py:263,266 fused with the act_quant of that GEMM, emitting codes
  */
 #ifndef FPQ_B200_H
 #define FPQ_B200_H
@@ -291,6 +292,24 @@ FPQ_API int fpq_unpack_codes(const uint8_t *codes, const float *scales, size_t r
  * non-negative half grid; byte i of `nibbles` holds codes 2i (low nibble) and 2i+1.  n_codes % 8 == 0.  Lossless both ways. */
 FPQ_API int fpq_codes_to_nibbles(const uint8_t *codes, size_t n_codes, int format, uint8_t *nibbles, void *stream);
 FPQ_API int fpq_nibbles_to_codes(const uint8_t *nibbles, size_t n_codes, int format, uint8_t *codes, void *stream);
+/*
+ * The fused activation path straight to codes: fpq_transform_rotate_quant / fpq_modulate_transform_rotate_quant with the
+ * quantized tensor emitted as an operand of fpq_gemm_codes (scale_group = 128) instead of as fp16, in ONE launch (padding rows
+ * included): 4 bytes read and 1 + 4/128 written per element, instead of the fp16 rotation (4 + 2) followed by fpq_pack_codes
+ * (2 + 1 + 1/32).  Arguments, alignment rules, FPQ_MOD_GAIN, the kernel tie rule and the choice between the small-launch and
+ * the streaming kernel are those of the fp16 siblings, except:
+ *   codes  : rows_pad * n_cols bytes in the layout above, 16-byte aligned (rows_pad = fpq_codes_rows_padded(n_rows))
+ *   scales : fp32 [n_cols/128][rows_pad], 4-byte aligned; each an fp16-rounded value, as fpq_pack_codes stores for fp16 input
+ *   format : FPQ_FMT_* (no -1: there is nothing to pack without a quantizer)
+ * Numerics contract: codes and scales are bit-identical to fpq_pack_codes(rotated, n_rows, n_cols, 128, FPQ_F16, format), where
+ * `rotated` is the fp16 output of the sibling call with format = -1; equivalently, fpq_unpack_codes of them to fp16 is
+ * bit-identical to the sibling's fake-quantized output.
+ */
+FPQ_API int fpq_transform_rotate_pack_codes(const float *x, const float *smooth, const uint32_t *sign_bits_host,
+                   uint8_t *codes, float *scales, size_t n_rows, size_t n_cols, int format, void *stream);
+FPQ_API int fpq_modulate_transform_rotate_pack_codes(const float *x, const float *scale, const float *shift, size_t rows_per_batch,
+                   const float *smooth, const uint32_t *sign_bits_host, uint8_t *codes, float *scales,
+                   size_t n_rows, size_t n_cols, int format, int flags, void *stream);
 /*
  * F.linear(A, W, bias) for A = [m, k] and W = [n, k] given as codes that share `scale_group` (128 or k):
  *   C[i, j] = bias[j] + fma-chain over the scale groups t (ascending) of  (P_t[i, j] * sa[t, i]) * sw[t, j],
