@@ -1,5 +1,6 @@
 // Shared device helpers of libfpq_b200 (constant grid tables, streaming loads/stores, the
-// 16-elements-per-lane register tile, group reductions, launch bookkeeping).
+// 16-elements-per-lane register tile, group reductions, launch bookkeeping) and the format
+// traits and run-time format / dtype dispatchers of every launcher.
 //
 // Thread mapping of the group kernels: a group of GS contiguous elements is owned by
 // LPG = GS/16 adjacent lanes; lane l holds 16 elements as 16-byte vectors, vector j of lane l
@@ -12,6 +13,7 @@
 #include <stddef.h>
 #include <stdlib.h>
 #include <math.h>
+#include <type_traits>
 
 #include "../../include/fpq_b200.h"
 #include "fpq_round.cuh"
@@ -117,6 +119,26 @@ static inline unsigned resident_row_grid(KernelT kernel, int threads, size_t n_r
     const size_t cap = size_t(sm_count()) * per_sm;
     return unsigned(n_rows < cap ? n_rows : cap);
 }
+// Launches a row-in-registers kernel (x, out, n_rows, row_vecs, last) on rows the caller has found eligible;
+// kernel_for(std::integral_constant<int, V>{}) returns the kernel for V = 1 | 2 | 4.  The occupancy cache is a static of
+// this template, so it stays per kernel family as long as each caller instantiation passes its own lambda type: residency
+// depends on each kernel's registers.
+template <typename KernelFor, typename InT, typename OutT, typename Last>
+static inline void launch_row_reg(KernelFor kernel_for, bool heavy_loop, const InT* x, OutT* out, size_t n_rows, size_t row_len, Last last,
+                                  cudaStream_t st) {
+    const size_t row_vecs = row_len / (16 / sizeof(InT));
+    const int v = row_reg_vectors(row_vecs, heavy_loop);
+    int threads = int((row_vecs + v - 1) / v);
+    threads = (threads + 31) / 32 * 32;
+    static int occ[3][33];                            // resident CTAs per SM, per (V, threads / 32); 0 = not asked yet
+    auto launch = [&](auto vc, int* cache) {
+        const auto k = kernel_for(vc);
+        k<<<resident_row_grid(k, threads, n_rows, cache), threads, 0, st>>>(x, out, n_rows, int(row_vecs), last);
+    };
+    if (v == 1) launch(std::integral_constant<int, 1>{}, occ[0]);
+    else if (v == 2) launch(std::integral_constant<int, 2>{}, occ[1]);
+    else launch(std::integral_constant<int, 4>{}, occ[2]);
+}
 
 // ------------------------------------------------------------------------------------------
 // Programmatic dependent launch (PDL).  The activation kernels are short (2-130 us) and a VAR pass
@@ -140,10 +162,10 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 void prefer_carveout(const void* kernel);
 
 template <typename... KArgs, typename... Args>
-static inline void launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t st, Args... args) {
+static inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, unsigned block, size_t smem, cudaStream_t st, Args... args) {
     prefer_carveout(reinterpret_cast<const void*>(kernel));
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
+    cfg.gridDim = grid;
     cfg.blockDim = dim3(block);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
@@ -272,12 +294,55 @@ __device__ __forceinline__ float group_max(float a) {      // NaN-ignoring (inpu
     return a;
 }
 
+// ------------------------------------------------------------------------------------------
+// The quantizer formats: the half grid and grid table of each symmetric format, the negative and
+// positive halves of each sign-split format, and the dispatchers that turn a run-time FPQ_FMT_* /
+// FPQ_SPLIT_* / dtype code into a template argument.  f receives a std::integral_constant (read
+// fmt.value) or a DType tag (read typename decltype(t)::type); a code outside the set is FPQ_ERR_ARG.
+// ------------------------------------------------------------------------------------------
 template <int FMT> struct SymFmt;
 template <> struct SymFmt<FPQ_FMT_E2M1> { using HG = HG_E2M1; static constexpr int GT = GT_E2M1; };
 template <> struct SymFmt<FPQ_FMT_E1M2> { using HG = HG_E1M2; static constexpr int GT = GT_E1M2; };
 template <> struct SymFmt<FPQ_FMT_E3M0> { using HG = HG_E3M0; static constexpr int GT = GT_E3M0; };
 template <> struct SymFmt<FPQ_FMT_E2M3> { using HG = HG_E2M3; static constexpr int GT = GT_E2M3; };
 template <> struct SymFmt<FPQ_FMT_E3M2> { using HG = HG_E3M2; static constexpr int GT = GT_E3M2; };
+
+template <int SPLIT> struct SplitFmt;
+template <> struct SplitFmt<FPQ_SPLIT_E1M2NEG_E2M1POS> { using NEG = HG_E1M2; using POS = HG_E2M1; static constexpr int GT_N = GT_E1M2_NEG, GT_P = GT_E2M1_POS; };
+template <> struct SplitFmt<FPQ_SPLIT_INTNEG_E2M3POS> { using NEG = HG_INT32; using POS = HG_E2M3; static constexpr int GT_N = GT_INT_NEG, GT_P = GT_E2M3_POS; };
+template <> struct SplitFmt<FPQ_SPLIT_AFPQ_E2M1> { using NEG = HG_E2M1; using POS = HG_E2M1; static constexpr int GT_N = GT_E2M1_NEG, GT_P = GT_E2M1_POS; };
+
+template <typename F>
+static inline int with_sym_format(int format, F&& f) {
+    switch (format) {
+        case FPQ_FMT_E2M1: return f(std::integral_constant<int, FPQ_FMT_E2M1>{});
+        case FPQ_FMT_E1M2: return f(std::integral_constant<int, FPQ_FMT_E1M2>{});
+        case FPQ_FMT_E3M0: return f(std::integral_constant<int, FPQ_FMT_E3M0>{});
+        case FPQ_FMT_E2M3: return f(std::integral_constant<int, FPQ_FMT_E2M3>{});
+        case FPQ_FMT_E3M2: return f(std::integral_constant<int, FPQ_FMT_E3M2>{});
+        default: return FPQ_ERR_ARG;
+    }
+}
+
+template <typename F>
+static inline int with_split_format(int split, F&& f) {
+    switch (split) {
+        case FPQ_SPLIT_E1M2NEG_E2M1POS: return f(std::integral_constant<int, FPQ_SPLIT_E1M2NEG_E2M1POS>{});
+        case FPQ_SPLIT_INTNEG_E2M3POS: return f(std::integral_constant<int, FPQ_SPLIT_INTNEG_E2M3POS>{});
+        case FPQ_SPLIT_AFPQ_E2M1: return f(std::integral_constant<int, FPQ_SPLIT_AFPQ_E2M1>{});
+        default: return FPQ_ERR_ARG;
+    }
+}
+
+template <typename T> struct DType { using type = T; };
+template <typename F>
+static inline int with_dtypes(int in_dtype, int out_dtype, F&& f) {
+    if (in_dtype == FPQ_F32 && out_dtype == FPQ_F32) return f(DType<float>{}, DType<float>{});
+    if (in_dtype == FPQ_F32 && out_dtype == FPQ_F16) return f(DType<float>{}, DType<__half>{});
+    if (in_dtype == FPQ_F16 && out_dtype == FPQ_F16) return f(DType<__half>{}, DType<__half>{});
+    if (in_dtype == FPQ_F16 && out_dtype == FPQ_F32) return f(DType<__half>{}, DType<float>{});
+    return FPQ_ERR_ARG;
+}
 
 // Is the scale "regular", i.e. may the reciprocal-multiply fast path be used?
 //   fp32 tensors: 2^-100 <= s <= 2^100 (1/s and x*(1/s) stay normal)

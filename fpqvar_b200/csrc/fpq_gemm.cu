@@ -667,30 +667,20 @@ bool half_grid_e4m3(int format, NibbleLut& lut) {
 template <typename T>
 int launch_pack_rows(int format, const T* x, size_t rows, size_t rows_pad, size_t k, uint8_t* codes, float* scales, cudaStream_t st) {
     const unsigned grid = grid_for(rows_pad / 8, 8, 8);
-    switch (format) {
-        case FPQ_FMT_E2M1: pack_codes_row_kernel<T, HG_E2M1><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E1M2: pack_codes_row_kernel<T, HG_E1M2><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E3M0: pack_codes_row_kernel<T, HG_E3M0><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E2M3: pack_codes_row_kernel<T, HG_E2M3><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E3M2: pack_codes_row_kernel<T, HG_E3M2><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        default: return FPQ_ERR_ARG;
-    }
-    return finish_launch();
+    return with_sym_format(format, [&](auto fmt) {
+        pack_codes_row_kernel<T, typename SymFmt<fmt.value>::HG><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales);
+        return finish_launch();
+    });
 }
 
 template <typename T>
 int launch_pack(int format, const T* x, size_t rows, size_t rows_pad, size_t k, uint8_t* codes, float* scales, cudaStream_t st) {
     const size_t tasks = (k / GK) * (rows_pad / 8);
     const unsigned grid = grid_for(tasks, 8, 8);
-    switch (format) {
-        case FPQ_FMT_E2M1: pack_codes_kernel<T, HG_E2M1><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E1M2: pack_codes_kernel<T, HG_E1M2><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E3M0: pack_codes_kernel<T, HG_E3M0><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E2M3: pack_codes_kernel<T, HG_E2M3><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        case FPQ_FMT_E3M2: pack_codes_kernel<T, HG_E3M2><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales); break;
-        default: return FPQ_ERR_ARG;
-    }
-    return finish_launch();
+    return with_sym_format(format, [&](auto fmt) {
+        pack_codes_kernel<T, typename SymFmt<fmt.value>::HG><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales);
+        return finish_launch();
+    });
 }
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }

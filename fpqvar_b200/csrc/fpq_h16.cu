@@ -172,11 +172,6 @@ __global__ void __launch_bounds__(256) fake_quant_segments_h16_kernel(const __ha
 // ------------------------------------------------------------------------------------------
 // sign-split
 // ------------------------------------------------------------------------------------------
-template <int SPLIT> struct SplitH16;
-template <> struct SplitH16<FPQ_SPLIT_E1M2NEG_E2M1POS> { using NEG = HG_E1M2; using POS = HG_E2M1; static constexpr int GT_N = GT_E1M2_NEG, GT_P = GT_E2M1_POS; };
-template <> struct SplitH16<FPQ_SPLIT_INTNEG_E2M3POS> { using NEG = HG_INT32; using POS = HG_E2M3; static constexpr int GT_N = GT_INT_NEG, GT_P = GT_E2M3_POS; };
-template <> struct SplitH16<FPQ_SPLIT_AFPQ_E2M1> { using NEG = HG_E2M1; using POS = HG_E2M1; static constexpr int GT_N = GT_E2M1_NEG, GT_P = GT_E2M1_POS; };
-
 // Group maxima by integer order of the fp16 bit patterns (two elements per VIMNMX):
 //   signed 16-bit max   -> the largest positive value (bits < 0x8000 order like the values)
 //   unsigned 16-bit max -> 0x8000 | largest negative magnitude, if any element is negative
@@ -185,7 +180,7 @@ template <> struct SplitH16<FPQ_SPLIT_AFPQ_E2M1> { using NEG = HG_E2M1; using PO
 // -> literal_split_nan_group_h16
 template <int SPLIT, int LPG, int NW>
 __device__ __forceinline__ int split_quant_tile_h16(uint32_t (&p)[NW], float& sn, float& sp, float delta) {
-    using SF = SplitH16<SPLIT>;
+    using SF = SplitFmt<SPLIT>;
     uint32_t pm = 0u, nm = 0u;
 #pragma unroll
     for (int i = 0; i < NW; ++i) { pm = __vmaxs2(pm, p[i]); nm = __vmaxu2(nm, p[i]); }
@@ -293,7 +288,7 @@ __global__ void __launch_bounds__(256) signsplit_group_h16_kernel(const __half* 
         }
     };
     auto work = [&](size_t gbase, uint32_t (&p)[H16_NW]) {
-        using SF = SplitH16<SPLIT>;
+        using SF = SplitFmt<SPLIT>;
         const size_t g = gbase + lane / H16_LPG;
         float sn, sp;
         const int rc = split_quant_tile_h16<SPLIT, H16_LPG, H16_NW>(p, sn, sp, delta);
@@ -325,30 +320,20 @@ int launch_sym_h16(int format, const void* x, void* out, size_t n_groups, cudaSt
     const __half* xi = static_cast<const __half*>(x);
     __half* oo = static_cast<__half*>(out);
     const unsigned grid = grid_h16(n_groups);
-    switch (format) {
-        case FPQ_FMT_E2M1: launch_pdl(fake_quant_group_h16_kernel<FPQ_FMT_E2M1>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E1M2: launch_pdl(fake_quant_group_h16_kernel<FPQ_FMT_E1M2>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E3M0: launch_pdl(fake_quant_group_h16_kernel<FPQ_FMT_E3M0>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E2M3: launch_pdl(fake_quant_group_h16_kernel<FPQ_FMT_E2M3>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E3M2: launch_pdl(fake_quant_group_h16_kernel<FPQ_FMT_E3M2>, grid, 256, 0, st, xi, oo, n_groups); break;
-        default: return FPQ_ERR_ARG;
-    }
-    return finish_launch();
+    return with_sym_format(format, [&](auto fmt) {
+        launch_pdl(fake_quant_group_h16_kernel<fmt.value>, grid, 256, 0, st, xi, oo, n_groups);
+        return finish_launch();
+    });
 }
 
 int launch_sym_h16_g64(int format, const void* x, void* out, size_t n_groups, cudaStream_t st) {
     const __half* xi = static_cast<const __half*>(x);
     __half* oo = static_cast<__half*>(out);
     const unsigned grid = grid_for(n_groups, 8 * 8 * 2, 8);       // 8 warps x 8 groups x 2 tiles per block and trip
-    switch (format) {
-        case FPQ_FMT_E2M1: launch_pdl(fake_quant_group64_h16_kernel<FPQ_FMT_E2M1>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E1M2: launch_pdl(fake_quant_group64_h16_kernel<FPQ_FMT_E1M2>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E3M0: launch_pdl(fake_quant_group64_h16_kernel<FPQ_FMT_E3M0>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E2M3: launch_pdl(fake_quant_group64_h16_kernel<FPQ_FMT_E2M3>, grid, 256, 0, st, xi, oo, n_groups); break;
-        case FPQ_FMT_E3M2: launch_pdl(fake_quant_group64_h16_kernel<FPQ_FMT_E3M2>, grid, 256, 0, st, xi, oo, n_groups); break;
-        default: return FPQ_ERR_ARG;
-    }
-    return finish_launch();
+    return with_sym_format(format, [&](auto fmt) {
+        launch_pdl(fake_quant_group64_h16_kernel<fmt.value>, grid, 256, 0, st, xi, oo, n_groups);
+        return finish_launch();
+    });
 }
 
 template <bool GELU>
@@ -356,13 +341,10 @@ static int launch_split_h16_t(int split, const void* x, void* out, size_t n_grou
     const __half* xi = static_cast<const __half*>(x);
     __half* oo = static_cast<__half*>(out);
     const unsigned grid = grid_h16(n_groups);
-    switch (split) {
-        case FPQ_SPLIT_E1M2NEG_E2M1POS: launch_pdl(signsplit_group_h16_kernel<FPQ_SPLIT_E1M2NEG_E2M1POS, GELU>, grid, 256, 0, st, xi, oo, n_groups, nan_flag); break;
-        case FPQ_SPLIT_INTNEG_E2M3POS: launch_pdl(signsplit_group_h16_kernel<FPQ_SPLIT_INTNEG_E2M3POS, GELU>, grid, 256, 0, st, xi, oo, n_groups, nan_flag); break;
-        case FPQ_SPLIT_AFPQ_E2M1: launch_pdl(signsplit_group_h16_kernel<FPQ_SPLIT_AFPQ_E2M1, GELU>, grid, 256, 0, st, xi, oo, n_groups, nan_flag); break;
-        default: return FPQ_ERR_ARG;
-    }
-    return finish_launch();
+    return with_split_format(split, [&](auto sf) {
+        launch_pdl(signsplit_group_h16_kernel<sf.value, GELU>, grid, 256, 0, st, xi, oo, n_groups, nan_flag);
+        return finish_launch();
+    });
 }
 int launch_split_h16(int split, const void* x, void* out, size_t n_groups, unsigned* nan_flag, cudaStream_t st) {
     return launch_split_h16_t<false>(split, x, out, n_groups, nan_flag, st);
@@ -421,7 +403,7 @@ __global__ void selftest_f16_flow_kernel(unsigned long long* result) {
             want[0] = f2h(quant_elem_literal<__half, TIE_KERNEL>(x, s, c_grids[SymFmt<CODE>::GT]) * s);
             want[1] = f2h(quant_elem_literal<__half, TIE_KERNEL>(-x, s, c_grids[SymFmt<CODE>::GT]) * s);
         } else {
-            using SF = SplitH16<CODE - 16>;
+            using SF = SplitFmt<CODE - 16>;
             // the other side's scale does not influence an element: use the same s on both sides
             got = split_pair_h16<typename SF::NEG, typename SF::POS>(x2, make_splitk<typename SF::NEG, typename SF::POS>(s, r, s, r), delta);
 #pragma unroll
@@ -449,7 +431,7 @@ __global__ void selftest_f16_flow_kernel(unsigned long long* result) {
             using HG = typename SymFmt<(CODE >= 32 ? CODE - 32 : CODE)>::HG;
             ok = same(__half_as_ushort(scale_from_absmax_h16<HG>(a)), f2h(__fdiv_rn(a, HG::VMAX)));
         } else {
-            using SF = SplitH16<CODE - 16>;
+            using SF = SplitFmt<CODE - 16>;
             ok = same(__half_as_ushort(scale_from_absmax_h16<typename SF::NEG>(a)), f2h(__fdiv_rn(a, SF::NEG::VMAX))) &&
                  same(__half_as_ushort(scale_from_absmax_h16<typename SF::POS>(a)), f2h(__fdiv_rn(a, SF::POS::VMAX)));
         }
@@ -494,24 +476,11 @@ static int launch_segments_h16(int format, const __half* x, __half* out, size_t 
     const size_t cap = (size_t(sm_count()) * 8 + n_segments - 1) / n_segments;
     if (per_seg > cap) per_seg = cap;
     if (per_seg < 1) per_seg = 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(unsigned(per_seg), unsigned(n_segments), 1);
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = g_tun.pdl ? 1 : 0;
-    switch (format) {
-        case FPQ_FMT_E2M1: cudaLaunchKernelEx(&cfg, fake_quant_segments_h16_kernel<FPQ_FMT_E2M1, GS>, x, out, groups_per_segment, pitch_x, pitch_out); break;
-        case FPQ_FMT_E1M2: cudaLaunchKernelEx(&cfg, fake_quant_segments_h16_kernel<FPQ_FMT_E1M2, GS>, x, out, groups_per_segment, pitch_x, pitch_out); break;
-        case FPQ_FMT_E3M0: cudaLaunchKernelEx(&cfg, fake_quant_segments_h16_kernel<FPQ_FMT_E3M0, GS>, x, out, groups_per_segment, pitch_x, pitch_out); break;
-        case FPQ_FMT_E2M3: cudaLaunchKernelEx(&cfg, fake_quant_segments_h16_kernel<FPQ_FMT_E2M3, GS>, x, out, groups_per_segment, pitch_x, pitch_out); break;
-        case FPQ_FMT_E3M2: cudaLaunchKernelEx(&cfg, fake_quant_segments_h16_kernel<FPQ_FMT_E3M2, GS>, x, out, groups_per_segment, pitch_x, pitch_out); break;
-        default: return FPQ_ERR_ARG;
-    }
-    return finish_launch();
+    const dim3 grid(unsigned(per_seg), unsigned(n_segments), 1);
+    return with_sym_format(format, [&](auto fmt) {
+        launch_pdl(fake_quant_segments_h16_kernel<fmt.value, GS>, grid, 256, 0, st, x, out, groups_per_segment, pitch_x, pitch_out);
+        return finish_launch();
+    });
 }
 
 extern "C" int fpq_fake_quant_segments(const void* x, void* out, size_t n_segments, size_t rows_per_segment, size_t row_len, size_t pitch_x,

@@ -704,16 +704,10 @@ static int launch_rotate(const float* x, const Modulate* mod, const float* smoot
     SignMask sm;
     for (int i = 0; i < 4; ++i) sm.w[i] = sign_bits_host[i];
     const int cpr = int(n_cols / 128);
-    switch (format) {
-        case FPQ_FMT_E2M1: return launch_fmt<FPQ_FMT_E2M1, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
-        case FPQ_FMT_E1M2: return launch_fmt<FPQ_FMT_E1M2, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
-        case FPQ_FMT_E3M0: return launch_fmt<FPQ_FMT_E3M0, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
-        case FPQ_FMT_E2M3: return launch_fmt<FPQ_FMT_E2M3, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
-        case FPQ_FMT_E3M2: return launch_fmt<FPQ_FMT_E3M2, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
-        default: break;
+    if constexpr (!CODES) {
+        if (format == -1) return launch_fmt<0, false, false>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
     }
-    if constexpr (!CODES) return launch_fmt<0, false, false>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st);
-    return FPQ_ERR_ARG;
+    return with_sym_format(format, [&](auto fmt) { return launch_fmt<fmt.value, true, CODES>(x, mod, smooth, sm, o, rot, co, n_rows, cpr, st); });
 }
 
 static int launch_rotate_quant(const float* x, const Modulate* mod, const float* smooth, const uint32_t* sign_bits_host, void* out, void* rotated,

@@ -12,11 +12,6 @@ namespace fpq {
 constexpr int MAX_CAND = 8;
 struct Candidates { int n; int fmt[MAX_CAND]; };
 
-template <int SPLIT> struct SplitFmtS;
-template <> struct SplitFmtS<FPQ_SPLIT_E1M2NEG_E2M1POS> { using NEG = HG_E1M2; using POS = HG_E2M1; static constexpr int GT_N = GT_E1M2_NEG, GT_P = GT_E2M1_POS; };
-template <> struct SplitFmtS<FPQ_SPLIT_INTNEG_E2M3POS> { using NEG = HG_INT32; using POS = HG_E2M3; static constexpr int GT_N = GT_INT_NEG, GT_P = GT_E2M3_POS; };
-template <> struct SplitFmtS<FPQ_SPLIT_AFPQ_E2M1> { using NEG = HG_E2M1; using POS = HG_E2M1; static constexpr int GT_N = GT_E2M1_NEG, GT_P = GT_E2M1_POS; };
-
 // squared error of one symmetric candidate over the lane's 16 values
 template <typename InT, int FMT, int TIE>
 __device__ __forceinline__ float sse_sym(const float (&v)[16], float a) {
@@ -49,7 +44,7 @@ __device__ __forceinline__ float sse_sym(const float (&v)[16], float a) {
 
 template <typename InT, int SPLIT, int TIE>
 __device__ __forceinline__ float sse_split(const float (&v)[16], float an, float ap) {
-    using SF = SplitFmtS<SPLIT>;
+    using SF = SplitFmt<SPLIT>;
     const float sn = rnd_in<InT>(__fdiv_rn(an, SF::NEG::VMAX));
     const float sp = rnd_in<InT>(__fdiv_rn(ap, SF::POS::VMAX));
     const bool n_ok = scale_regular<InT>(sn) || (TIE == TIE_KERNEL && sn == 0.0f);
@@ -227,7 +222,7 @@ __device__ __forceinline__ float sse_sym_h16(const uint32_t (&p)[16], const uint
 
 template <int SPLIT>
 __device__ __forceinline__ float sse_split_h16(const uint32_t (&p)[16], const uint64_t (&xf)[16], uint32_t pbits, uint32_t nbits, float delta, const __half* src, int lig) {
-    using SF = SplitFmtS<SPLIT>;
+    using SF = SplitFmt<SPLIT>;
     const float an = h2f(uint16_t(nbits)), ap = h2f(uint16_t(pbits));
     const __half snh = scale_from_absmax_h16<typename SF::NEG>(an), sph = scale_from_absmax_h16<typename SF::POS>(ap);
     const bool fast = (scale_bits_regular(__half_as_ushort(snh)) || nbits == 0u) && (scale_bits_regular(__half_as_ushort(sph)) || pbits == 0u);

@@ -7,11 +7,6 @@ namespace fpq {
 // ------------------------------------------------------------------------------------------
 // Sign-split formats
 // ------------------------------------------------------------------------------------------
-template <int SPLIT> struct SplitFmt;
-template <> struct SplitFmt<FPQ_SPLIT_E1M2NEG_E2M1POS> { using NEG = HG_E1M2; using POS = HG_E2M1; static constexpr int GT_N = GT_E1M2_NEG, GT_P = GT_E2M1_POS; };
-template <> struct SplitFmt<FPQ_SPLIT_INTNEG_E2M3POS> { using NEG = HG_INT32; using POS = HG_E2M3; static constexpr int GT_N = GT_INT_NEG, GT_P = GT_E2M3_POS; };
-template <> struct SplitFmt<FPQ_SPLIT_AFPQ_E2M1> { using NEG = HG_E2M1; using POS = HG_E2M1; static constexpr int GT_N = GT_E2M1_NEG, GT_P = GT_E2M1_POS; };
-
 // One element, literal reference sequence (quant_utils.py:428-451 / :404-410).
 template <typename InT, typename OutT, int SPLIT, int TIE>
 __device__ __forceinline__ float signsplit_elem_literal(float x, float sn, float sp) {
@@ -301,28 +296,12 @@ __global__ void __launch_bounds__(1024) signsplit_row_reg_kernel(const InT* __re
     }
 }
 
-template <typename InT, typename OutT, int SPLIT, int TIE>
-static bool launch_split_row_reg(const InT* xi, OutT* oo, size_t n_rows, size_t row_len, unsigned* flag, cudaStream_t st) {
+template <typename InT, typename OutT>
+static bool split_row_reg_fits(const InT* xi, OutT* oo, size_t row_len) {
     constexpr int VEC = 16 / sizeof(InT);
     if (row_len % VEC != 0 || row_len < 256) return false;
     if ((reinterpret_cast<uintptr_t>(xi) & 15) || (reinterpret_cast<uintptr_t>(oo) & 15)) return false;
-    const size_t row_vecs = row_len / VEC;
-    if (row_vecs > 4096) return false;
-    const int v = row_reg_vectors(row_vecs, true);
-    int threads = int((row_vecs + v - 1) / v);
-    threads = (threads + 31) / 32 * 32;
-    static int occ[3][33];                            // resident CTAs per SM, per (V, threads / 32); 0 = not asked yet
-    if (v == 1) {
-        auto k = signsplit_row_reg_kernel<InT, OutT, SPLIT, TIE, 1>;
-        k<<<resident_row_grid(k, threads, n_rows, occ[0]), threads, 0, st>>>(xi, oo, n_rows, int(row_vecs), flag);
-    } else if (v == 2) {
-        auto k = signsplit_row_reg_kernel<InT, OutT, SPLIT, TIE, 2>;
-        k<<<resident_row_grid(k, threads, n_rows, occ[1]), threads, 0, st>>>(xi, oo, n_rows, int(row_vecs), flag);
-    } else {
-        auto k = signsplit_row_reg_kernel<InT, OutT, SPLIT, TIE, 4>;
-        k<<<resident_row_grid(k, threads, n_rows, occ[2]), threads, 0, st>>>(xi, oo, n_rows, int(row_vecs), flag);
-    }
-    return true;
+    return row_len / VEC <= 4096;
 }
 
 // qu.py:421-422 with a NaN in the tensor: clamp(x, -NaN, NaN) makes every element NaN, both
@@ -358,7 +337,9 @@ static int launch_split(const void* x, void* out, size_t n_rows, size_t row_len,
         const unsigned grid = grid_for(n_rows, groups_per_block, 64);
         if (lpg == 8) signsplit_group_kernel<InT, OutT, SPLIT, TIE, 8><<<grid, 256, 0, st>>>(xi, oo, n_rows, flag);
         else signsplit_group_kernel<InT, OutT, SPLIT, TIE, 4><<<grid, 256, 0, st>>>(xi, oo, n_rows, flag);
-    } else if (!launch_split_row_reg<InT, OutT, SPLIT, TIE>(xi, oo, n_rows, row_len, flag, st)) {
+    } else if (split_row_reg_fits(xi, oo, row_len)) {
+        launch_row_reg([](auto v) { return signsplit_row_reg_kernel<InT, OutT, SPLIT, TIE, v.value>; }, true, xi, oo, n_rows, row_len, flag, st);
+    } else {
         const unsigned grid = grid_for(n_rows, 1, 16);
         signsplit_row_kernel<InT, OutT, SPLIT, TIE><<<grid, 256, 0, st>>>(xi, oo, n_rows, row_len, flag);
     }
@@ -373,36 +354,26 @@ static int launch_split(const void* x, void* out, size_t n_rows, size_t row_len,
     return finish_launch();
 }
 
-template <typename InT, typename OutT, int TIE>
-static int dispatch_split_fmt(int split, const void* x, void* out, size_t n_rows, size_t row_len, unsigned* flag, cudaStream_t st) {
-    switch (split) {
-        case FPQ_SPLIT_E1M2NEG_E2M1POS: return launch_split<InT, OutT, FPQ_SPLIT_E1M2NEG_E2M1POS, TIE>(x, out, n_rows, row_len, flag, st);
-        case FPQ_SPLIT_INTNEG_E2M3POS: return launch_split<InT, OutT, FPQ_SPLIT_INTNEG_E2M3POS, TIE>(x, out, n_rows, row_len, flag, st);
-        case FPQ_SPLIT_AFPQ_E2M1: return launch_split<InT, OutT, FPQ_SPLIT_AFPQ_E2M1, TIE>(x, out, n_rows, row_len, flag, st);
-        default: return FPQ_ERR_ARG;
-    }
-}
-
 template <int TIE>
-static int dispatch_split_types(int in_dtype, int out_dtype, int split, const void* x, void* out, size_t n_rows, size_t row_len,
-                                unsigned* flag, cudaStream_t st) {
-    if (in_dtype == FPQ_F32 && out_dtype == FPQ_F32) return dispatch_split_fmt<float, float, TIE>(split, x, out, n_rows, row_len, flag, st);
-    if (in_dtype == FPQ_F16 && out_dtype == FPQ_F16) return dispatch_split_fmt<__half, __half, TIE>(split, x, out, n_rows, row_len, flag, st);
-    if (in_dtype == FPQ_F16 && out_dtype == FPQ_F32) return dispatch_split_fmt<__half, float, TIE>(split, x, out, n_rows, row_len, flag, st);
-    if (in_dtype == FPQ_F32 && out_dtype == FPQ_F16) return dispatch_split_fmt<float, __half, TIE>(split, x, out, n_rows, row_len, flag, st);
-    return FPQ_ERR_ARG;
+static int dispatch_split(int in_dtype, int out_dtype, int split, const void* x, void* out, size_t n_rows, size_t row_len, unsigned* flag,
+                          cudaStream_t st) {
+    return with_dtypes(in_dtype, out_dtype, [&](auto in_t, auto out_t) {
+        return with_split_format(split, [&](auto sf) {
+            return launch_split<typename decltype(in_t)::type, typename decltype(out_t)::type, sf.value, TIE>(x, out, n_rows, row_len, flag, st);
+        });
+    });
 }
 
 // One translation unit per tie rule (FPQ_SPLIT_TIE_PART = 0 / 1: fpq_split_k.cu / fpq_split_a.cu), as for fpq_sym.
 #if FPQ_SPLIT_TIE_PART == 0
 int signsplit_kernel_tie(int in_dtype, int out_dtype, int split, const void* x, void* out, size_t n_rows, size_t row_len, unsigned* flag,
                          cudaStream_t st) {
-    return dispatch_split_types<TIE_KERNEL>(in_dtype, out_dtype, split, x, out, n_rows, row_len, flag, st);
+    return dispatch_split<TIE_KERNEL>(in_dtype, out_dtype, split, x, out, n_rows, row_len, flag, st);
 }
 #else
 int signsplit_argmin_tie(int in_dtype, int out_dtype, int split, const void* x, void* out, size_t n_rows, size_t row_len, unsigned* flag,
                          cudaStream_t st) {
-    return dispatch_split_types<TIE_ARGMIN>(in_dtype, out_dtype, split, x, out, n_rows, row_len, flag, st);
+    return dispatch_split<TIE_ARGMIN>(in_dtype, out_dtype, split, x, out, n_rows, row_len, flag, st);
 }
 #endif
 

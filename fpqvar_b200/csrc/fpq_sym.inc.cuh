@@ -215,31 +215,15 @@ __global__ void __launch_bounds__(1024) fake_quant_row_reg_kernel(const InT* __r
     }
 }
 
-template <typename InT, typename OutT, int FMT, int TIE>
-static bool launch_row_reg(const InT* xi, OutT* oo, size_t n_rows, size_t row_len, int clamp3, cudaStream_t st) {
+template <typename InT, typename OutT>
+static bool sym_row_reg_fits(const InT* xi, OutT* oo, size_t row_len) {
     constexpr int VEC = 16 / sizeof(InT);
     if (row_len % VEC != 0 || row_len < 256) return false;
     if ((reinterpret_cast<uintptr_t>(xi) & 15) || (reinterpret_cast<uintptr_t>(oo) & 15)) return false;
     if ((row_len * sizeof(OutT)) % 16 != 0 && sizeof(OutT) < sizeof(InT)) {
         if ((row_len * sizeof(OutT)) % 8 != 0) return false;
     }
-    const size_t row_vecs = row_len / VEC;
-    if (row_vecs > 4096) return false;
-    const int v = row_reg_vectors(row_vecs, false);
-    int threads = int((row_vecs + v - 1) / v);
-    threads = (threads + 31) / 32 * 32;
-    static int occ[3][33];                            // resident CTAs per SM, per (V, threads / 32); 0 = not asked yet
-    if (v == 1) {
-        auto k = fake_quant_row_reg_kernel<InT, OutT, FMT, TIE, 1>;
-        k<<<resident_row_grid(k, threads, n_rows, occ[0]), threads, 0, st>>>(xi, oo, n_rows, int(row_vecs), clamp3);
-    } else if (v == 2) {
-        auto k = fake_quant_row_reg_kernel<InT, OutT, FMT, TIE, 2>;
-        k<<<resident_row_grid(k, threads, n_rows, occ[1]), threads, 0, st>>>(xi, oo, n_rows, int(row_vecs), clamp3);
-    } else {
-        auto k = fake_quant_row_reg_kernel<InT, OutT, FMT, TIE, 4>;
-        k<<<resident_row_grid(k, threads, n_rows, occ[2]), threads, 0, st>>>(xi, oo, n_rows, int(row_vecs), clamp3);
-    }
-    return true;
+    return row_len / VEC <= 4096;
 }
 
 template <typename InT, typename OutT, int FMT, int TIE>
@@ -258,33 +242,23 @@ static int launch_sym(const void* x, void* out, size_t n_rows, size_t row_len, i
         const unsigned grid = grid_for(n_rows, groups_per_block, 64);
         if (lpg == 8) fake_quant_group_kernel<InT, OutT, FMT, TIE, 8><<<grid, 256, 0, st>>>(xi, oo, n_rows, clamp3);
         else fake_quant_group_kernel<InT, OutT, FMT, TIE, 4><<<grid, 256, 0, st>>>(xi, oo, n_rows, clamp3);
-    } else if (!launch_row_reg<InT, OutT, FMT, TIE>(xi, oo, n_rows, row_len, clamp3, st)) {
+    } else if (sym_row_reg_fits(xi, oo, row_len)) {
+        launch_row_reg([](auto v) { return fake_quant_row_reg_kernel<InT, OutT, FMT, TIE, v.value>; }, false, xi, oo, n_rows, row_len, clamp3, st);
+    } else {
         const unsigned grid = grid_for(n_rows, 1, 16);
         fake_quant_row_kernel<InT, OutT, FMT, TIE><<<grid, 256, 0, st>>>(xi, oo, n_rows, row_len, clamp3);
     }
     return finish_launch();
 }
 
-template <typename InT, typename OutT, int TIE>
-static int dispatch_sym_fmt(int format, const void* x, void* out, size_t n_rows, size_t row_len, int clamp3, cudaStream_t st) {
-    switch (format) {
-        case FPQ_FMT_E2M1: return launch_sym<InT, OutT, FPQ_FMT_E2M1, TIE>(x, out, n_rows, row_len, clamp3, st);
-        case FPQ_FMT_E1M2: return launch_sym<InT, OutT, FPQ_FMT_E1M2, TIE>(x, out, n_rows, row_len, clamp3, st);
-        case FPQ_FMT_E3M0: return launch_sym<InT, OutT, FPQ_FMT_E3M0, TIE>(x, out, n_rows, row_len, clamp3, st);
-        case FPQ_FMT_E2M3: return launch_sym<InT, OutT, FPQ_FMT_E2M3, TIE>(x, out, n_rows, row_len, clamp3, st);
-        case FPQ_FMT_E3M2: return launch_sym<InT, OutT, FPQ_FMT_E3M2, TIE>(x, out, n_rows, row_len, clamp3, st);
-        default: return FPQ_ERR_ARG;
-    }
-}
-
 template <int TIE>
-static int dispatch_sym_types(int in_dtype, int out_dtype, int format, const void* x, void* out, size_t n_rows, size_t row_len,
-                              int clamp3, cudaStream_t st) {
-    if (in_dtype == FPQ_F32 && out_dtype == FPQ_F32) return dispatch_sym_fmt<float, float, TIE>(format, x, out, n_rows, row_len, clamp3, st);
-    if (in_dtype == FPQ_F32 && out_dtype == FPQ_F16) return dispatch_sym_fmt<float, __half, TIE>(format, x, out, n_rows, row_len, clamp3, st);
-    if (in_dtype == FPQ_F16 && out_dtype == FPQ_F16) return dispatch_sym_fmt<__half, __half, TIE>(format, x, out, n_rows, row_len, clamp3, st);
-    if (in_dtype == FPQ_F16 && out_dtype == FPQ_F32) return dispatch_sym_fmt<__half, float, TIE>(format, x, out, n_rows, row_len, clamp3, st);
-    return FPQ_ERR_ARG;
+static int dispatch_sym(int in_dtype, int out_dtype, int format, const void* x, void* out, size_t n_rows, size_t row_len, int clamp3,
+                        cudaStream_t st) {
+    return with_dtypes(in_dtype, out_dtype, [&](auto in_t, auto out_t) {
+        return with_sym_format(format, [&](auto fmt) {
+            return launch_sym<typename decltype(in_t)::type, typename decltype(out_t)::type, fmt.value, TIE>(x, out, n_rows, row_len, clamp3, st);
+        });
+    });
 }
 
 // One translation unit per tie rule (FPQ_SYM_TIE_PART = 0 / 1, see fpq_sym_k.cu / fpq_sym_a.cu): the 4 dtype
@@ -292,12 +266,12 @@ static int dispatch_sym_types(int in_dtype, int out_dtype, int format, const voi
 #if FPQ_SYM_TIE_PART == 0
 int fake_quant_kernel_tie(int in_dtype, int out_dtype, int format, const void* x, void* out, size_t n_rows, size_t row_len, int clamp3,
                           cudaStream_t st) {
-    return dispatch_sym_types<TIE_KERNEL>(in_dtype, out_dtype, format, x, out, n_rows, row_len, clamp3, st);
+    return dispatch_sym<TIE_KERNEL>(in_dtype, out_dtype, format, x, out, n_rows, row_len, clamp3, st);
 }
 #else
 int fake_quant_argmin_tie(int in_dtype, int out_dtype, int format, const void* x, void* out, size_t n_rows, size_t row_len, int clamp3,
                           cudaStream_t st) {
-    return dispatch_sym_types<TIE_ARGMIN>(in_dtype, out_dtype, format, x, out, n_rows, row_len, clamp3, st);
+    return dispatch_sym<TIE_ARGMIN>(in_dtype, out_dtype, format, x, out, n_rows, row_len, clamp3, st);
 }
 #endif
 
