@@ -210,6 +210,14 @@ FPQ_API int fpq_transform_rotate_weight(const float *w, const float *smooth, con
  * reading x ONCE.  formats[] entries: FPQ_FMT_* (0..4) or 16+FPQ_SPLIT_* for sign-split
  * candidates; host array.  sse: n_formats doubles on the device, accumulated into (the caller
  * zeroes them and divides by the element count for the reference's mean).
+ * Accuracy: per-element errors are those of the fake quantizers (bit-exact); squares and partial sums are fp32 over lane
+ * pieces of one group (fp32 input: 16 elements, element i in piece (i / 4) % 8; fp16 input: 16 or 32 elements), then float64.
+ * The result is within 2e-6 relative of the float64 sum, plus n * 2^-149 for n scored elements: each fp32 rounding has an
+ * absolute error of up to 2^-150, so squares of errors below 2^-63 lose relative accuracy and those below 2^-75 count as 0
+ * (fp32 groups with an absmax below about 2^-60 all score 0).  A NaN, or an inf error, gives NaN or +inf as the float64
+ * sum of the reference's errors would.  fp32 overflow of the squares: if the float64 SSE of some piece exceeds 2 FLT_MAX the
+ * result is +inf (never NaN, never a finite number); if every piece's stays below FLT_MAX / 2 it is finite; between the two,
+ * fp32 rounding decides.  fp16 input reaches neither range.
  */
 FPQ_API int fpq_score_formats(const void *x, size_t n_rows, size_t row_len, int in_dtype,
                       const int *formats_host, int n_formats, int tie_mode,
@@ -233,6 +241,9 @@ FPQ_API int fpq_selftest_gelu(void *table_65536_halves, void *stream);
  * be NULL (= 1); out is one float64 accumulator the caller zeroes.  n_cols must fill whole 16-byte vectors.  Replaces
  * compute_quant_error(y_fp, y_q) = mean((y_fp - y_q)^2) inside the reference's search loop
  * (search/search_fp4_format.py:472-476, :798-816; search_fp6_format.py:807-868).
+ * Squares and partial sums are fp32 over pieces of at most 16 elements of a row, then float64 (times the row's weight): if the
+ * float64 SSE of some piece exceeds 2 FLT_MAX the result is +inf, if every piece's stays below FLT_MAX / 2 it is finite;
+ * squares below the fp32 range count as 0 (an absolute error of up to 2^-149 per element).  A NaN or inf anywhere gives the class (NaN / +inf) of the float64 sum, also in a row whose weight is 0.
  */
 FPQ_API int fpq_sse_rows(const void *a, const void *b, size_t n_rows, size_t n_cols, int dtype,
                    const double *row_weight, double *out, void *stream);
@@ -334,7 +345,10 @@ FPQ_API int fpq_gemm_codes(const uint8_t *a_codes, const float *a_scales, size_t
  *   *sse += sum_{i<m} row_weight[i] * sum_{j<n} (ref[i, j] - C[i, j])^2,   C as fpq_gemm_codes computes it in fp32 (never stored)
  * ref: [m, ldr] row-major, FPQ_F16 | FPQ_F32, the full-precision layer output; row_weight: float64 [m] or NULL (= 1): with the
  * calibration tensors stacked into one matrix, 1 / (rows_of_its_tensor * n * tensors) turns the sum into the reference's mean of
- * per-tensor means; sse: one float64 accumulator the caller zeroes.
+ * per-tensor means; sse: one float64 accumulator the caller zeroes.  Only columns [0, n) of rows [0, m) of ref are read.
+ * Squares and partial sums are fp32 over each thread's piece of a row (at most 32 products), then float64: if the float64
+ * SSE of some piece exceeds 2 FLT_MAX the result is +inf, if every piece's stays below FLT_MAX / 2 it is finite; squares
+ * below the fp32 range count as 0.
  */
 FPQ_API int fpq_gemm_codes_sse(const uint8_t *a_codes, const float *a_scales, size_t m, const uint8_t *b_codes,
                    const float *b_scales, size_t n, size_t k, size_t scale_group, const float *bias, int ref_dtype,
