@@ -32,6 +32,8 @@
 //   groups of 128 1.04-1.49 PFLOP/s: the epilogue's 2 flops per element (512 clk of the fp32 pipe per 128 x 256 slab, as long as
 //   the slab's MMAs) and its tensor-memory loads do not fully overlap with a memory-bound main loop; DESIGN.md 3.6 has the
 //   experiments (tcgen05.ld alone: ~1 KB/clk per SM, tools/tmem_ldbench.cu; epilogue compiled out; per-tile overhead).
+#include <atomic>
+
 #include "fpq_codes.cuh"
 #include "fpq_stream.cuh"
 
@@ -754,13 +756,14 @@ int launch_gemm(GemmArgs& g, cudaStream_t st) {
     if (tiles > 0x7fffffffull) return FPQ_ERR_UNSUPPORTED;
     g.n_tiles = uint32_t(tiles);
     g.tiles_n = uint32_t(tiles_n);
-    static bool attr_set[64] = {};
+    // per device: set once the attribute is; a thread that sees it set launches after the attribute call (release / acquire)
+    static std::atomic<bool> attr_set[64];
     int dev = 0;
     cudaGetDevice(&dev);
-    if (!attr_set[dev & 63]) {
+    if (!attr_set[dev & 63].load(std::memory_order_acquire)) {
         if (cudaFuncSetAttribute(gemm_codes_kernel<TN_, EC_, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(Cfg::smem_bytes(Cfg::MAX_STAGES))) != cudaSuccess)
             return finish_launch();
-        attr_set[dev & 63] = true;
+        attr_set[dev & 63].store(true, std::memory_order_release);
     }
     const size_t resident = size_t(sm_count());
     const unsigned grid = unsigned(tiles < resident ? tiles : resident);
@@ -779,8 +782,9 @@ int launch_gemm_pair(GemmArgs& g, cudaStream_t st) {
     g.n_tiles = uint32_t(tiles_m * tiles_n);
     g.tiles_n = uint32_t(tiles_n);
     auto kernel = gemm_codes_kernel<TN_, EC_, OUT, true>;
-    static bool attr_set[64] = {};
-    static int max_clusters[64] = {};
+    // per device: resident clusters, 0 = not known yet.  Published after the shared-memory attribute is set, in one atomic, so that
+    // a thread that reads a count also sees the attribute (two plain statics could be seen in either order: a grid of 0 clusters)
+    static std::atomic<int> max_clusters[64];
     int dev = 0;
     cudaGetDevice(&dev);
     cudaLaunchConfig_t cfg = {};
@@ -794,15 +798,14 @@ int launch_gemm_pair(GemmArgs& g, cudaStream_t st) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (!attr_set[dev & 63]) {
+    int n = max_clusters[dev & 63].load(std::memory_order_acquire);
+    if (n == 0) {
         if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(Cfg::smem_bytes_pair(Cfg::MAX_STAGES_PAIR))) != cudaSuccess) return finish_launch();
         cfg.gridDim = dim3(unsigned(sm_count()) / 2 * 2);
-        int n = 0;
         if (cudaOccupancyMaxActiveClusters(&n, kernel, &cfg) != cudaSuccess || n < 1) { cudaGetLastError(); n = sm_count() / 2 - 4; }
-        max_clusters[dev & 63] = n;
-        attr_set[dev & 63] = true;
+        max_clusters[dev & 63].store(n, std::memory_order_release);
     }
-    const size_t clusters = pairs < size_t(max_clusters[dev & 63]) ? pairs : size_t(max_clusters[dev & 63]);
+    const size_t clusters = pairs < size_t(n) ? pairs : size_t(n);
     cfg.gridDim = dim3(unsigned(2 * clusters));
     cudaLaunchKernelEx(&cfg, kernel, g);
     return finish_launch();

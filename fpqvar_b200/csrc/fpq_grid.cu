@@ -1,5 +1,6 @@
 // libfpq_b200 -- quant_cuda.quant compatibility entry (row a1), the exhaustive rounding self-test, and launch bookkeeping
 // Part of the C ABI of include/fpq_b200.h; no torch types here.
+#include <atomic>
 #include <cstdlib>
 #include <cstring>
 #include "fpq_common.cuh"
@@ -124,12 +125,14 @@ void prefer_carveout(const void* kernel) {
 int sm_count() {
     // per device ordinal (a process may drive several GPUs; the occupancy caches of the row kernels are per kernel only:
     // they depend on the kernel's registers and the architecture, and this library runs on B200s alone)
-    static int n[64] = {};
+    // 0 = not asked yet; the count is validated before it is published (another thread may read it at any time)
+    static std::atomic<int> n[64];
     int dev = 0;
     cudaGetDevice(&dev);
-    int& c = n[dev & 63];
+    int c = n[dev & 63].load(std::memory_order_relaxed);
     if (c == 0) {
         if (cudaDeviceGetAttribute(&c, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || c <= 0) c = 148;
+        n[dev & 63].store(c, std::memory_order_relaxed);
     }
     return c;
 }

@@ -15,6 +15,8 @@
 //   * a Sylvester Hadamard transform is the tensor product of a 2-point butterfly (a + b, a - b) over every
 //     index bit of the chunk position, in any order; the order fixes the fp32 summation tree and is
 //     0, 1, 5, 6, 2, 3, 4 in both kernels.
+#include <atomic>
+
 #include "fpq_codes.cuh"
 #include "fpq_stream.cuh"
 
@@ -639,12 +641,12 @@ static int launch_stream(const float* x, const float* smooth, const SignMask& sm
     if constexpr (MOD) kernel = modulate_transform_rotate_quant_stream_kernel<FMT, QUANT, CODES>;
     else kernel = transform_rotate_quant_stream_kernel<FMT, QUANT, CODES>;
     const size_t smem = size_t(plan.warps) * ROT_WARP_SMEM;
-    static bool attr_done[64] = {};                    // per instantiation and device
+    static std::atomic<bool> attr_done[64];           // per instantiation and device; set (release) after the attribute is
     int dev = 0;
     cudaGetDevice(&dev);
-    if (!attr_done[dev & 63]) {
+    if (!attr_done[dev & 63].load(std::memory_order_acquire)) {
         if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (ROT_MAX_CPR + 3) / 4 * ROT_WARP_SMEM) != cudaSuccess) return FPQ_ERR_CUDA;
-        attr_done[dev & 63] = true;
+        attr_done[dev & 63].store(true, std::memory_order_release);
     }
     const size_t steps = (n_rows + 1) / 2;
     const size_t cap = size_t(sm_count()) * plan.ctas_per_sm;
