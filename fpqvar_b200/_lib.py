@@ -64,6 +64,16 @@ SIGNATURES = {
                                   _c.c_size_t, _c.c_void_p, _c.c_int, _c.c_void_p, _c.c_size_t, _c.c_void_p]),
     "fpq_gemm_codes_sse": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_size_t,
                                       _c.c_size_t, _c.c_void_p, _c.c_int, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p, _c.c_void_p]),
+    "fpq_pack_codes_signsplit": (_c.c_int, [_c.c_void_p, _c.c_size_t, _c.c_size_t, _c.c_int, _c.c_int, _c.c_uint, _c.c_void_p,
+                                            _c.c_void_p, _c.c_void_p, _c.c_void_p]),
+    "fpq_gelu_pack_codes_signsplit": (_c.c_int, [_c.c_void_p, _c.c_size_t, _c.c_size_t, _c.c_int, _c.c_uint, _c.c_void_p,
+                                                 _c.c_void_p, _c.c_void_p, _c.c_void_p]),
+    "fpq_unpack_codes_signsplit": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_size_t, _c.c_int, _c.c_void_p, _c.c_void_p]),
+    "fpq_gemm_codes_signsplit": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_size_t,
+                                            _c.c_void_p, _c.c_int, _c.c_void_p, _c.c_size_t, _c.c_void_p]),
+    "fpq_gemm_codes_signsplit_sse": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p, _c.c_size_t,
+                                                _c.c_size_t, _c.c_void_p, _c.c_int, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p,
+                                                _c.c_void_p]),
 }
 
 _lib = None

@@ -186,6 +186,131 @@ __global__ void __launch_bounds__(256) unpack_codes_kernel(const uint8_t* __rest
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Sign-split operand (the fc2 input, qu.py:415-452): every 128-group t of a row has two scales, sn for x <= 0 and sp for x > 0,
+// and stands for qn * sn + qp * sp with one of qn, qp 0 in every element.  It is stored as a symmetric operand of depth 2k:
+// slab 2t holds the negative half's codes (0 where x > 0) with scale sn, slab 2t + 1 the positive half's (0 where x <= 0) with
+// scale sp.  Each half is the symmetric quantization of where(x <= 0, x, 0) (resp. where(x > 0, x, 0)) on the half's format:
+// its absmax is the half's own, and for values of one sign the nearest entry of the symmetric grid is the nearest entry of the
+// one-sided grid (ties go to the larger value on both), so grid_values16 of the half's trait (SplitFmt<>::NEG / POS) is the
+// reference's scan.  A NaN element counts as 0 on both sides (where()); nan_flag (FPQ_FLAG_GLOBAL_CLIP) records that the
+// tensor holds one.  Same mapping as pack_codes_kernel: one warp per (8 rows x 128 K) block of the input.
+// ---------------------------------------------------------------------------------------------------------------------
+template <typename T, int SPLIT, bool GELU>
+__global__ void __launch_bounds__(256) pack_codes_split_kernel(const T* __restrict__ x, size_t rows, size_t rows_pad, size_t k,
+                                                               uint8_t* __restrict__ codes, float* __restrict__ scales,
+                                                               unsigned* __restrict__ nan_flag) {
+    using SF = SplitFmt<SPLIT>;
+    const int lane = threadIdx.x & 31;
+    const int r = lane & 7, kq = lane >> 3;
+    const size_t slabs = k / GK, row_blocks = rows_pad / 8;
+    const size_t n_tasks = slabs * row_blocks;
+    const size_t warp0 = (size_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5, n_warps = (size_t(gridDim.x) * blockDim.x) >> 5;
+    for (size_t task = warp0; task < n_tasks; task += n_warps) {
+        const size_t rb = task / slabs, slab = task % slabs;
+        const size_t row = rb * 8 + r;
+        const bool live = row < rows;
+        float v[2][16];
+        float an = 0.0f, ap = 0.0f;
+        bool nan = false;
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            if (live) Chunk16<T>::load(x + row * k + slab * GK + size_t(kq + 4 * j) * 16, v[j]);
+            else {
+#pragma unroll
+                for (int i = 0; i < 16; ++i) v[j][i] = 0.0f;
+            }
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+                if constexpr (GELU) v[j][i] = __half2float(__float2half_rn(gelu_tanh_f32(v[j][i])));    // as gelu_tanh_h2
+                an = fmaxf(an, (v[j][i] <= 0.0f) ? -v[j][i] : 0.0f);
+                ap = fmaxf(ap, (v[j][i] > 0.0f) ? v[j][i] : 0.0f);
+                nan |= v[j][i] != v[j][i];
+            }
+        }
+        an = fmaxf(an, __shfl_xor_sync(0xffffffffu, an, 8));
+        an = fmaxf(an, __shfl_xor_sync(0xffffffffu, an, 16));
+        ap = fmaxf(ap, __shfl_xor_sync(0xffffffffu, ap, 8));
+        ap = fmaxf(ap, __shfl_xor_sync(0xffffffffu, ap, 16));
+        if (__any_sync(0xffffffffu, nan) && nan_flag != nullptr && lane == 0) atomicOr(nan_flag, 1u);
+        const float sn = Chunk16<T>::scale(an, SF::NEG::VMAX), sp = Chunk16<T>::scale(ap, SF::POS::VMAX);     // qu.py:432-433
+        uint8_t* blk_n = codes + (2 * slab * row_blocks + rb) * BLK_BYTES;
+        uint8_t* blk_p = blk_n + row_blocks * BLK_BYTES;
+        const float delta = tie_delta_kernel(uint32_t(uint64_t(task) >> 40));
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            float h[16], q[16];
+#pragma unroll
+            for (int i = 0; i < 16; ++i) h[i] = (v[j][i] <= 0.0f) ? v[j][i] : 0.0f;            // qu.py:428
+            grid_values16<T, typename SF::NEG>(h, sn, delta, q);
+            *reinterpret_cast<uint4*>(blk_n + (kq + 4 * j) * 128 + r * 16) =
+                make_uint4(e4m3x4(q[0], q[1], q[2], q[3]), e4m3x4(q[4], q[5], q[6], q[7]), e4m3x4(q[8], q[9], q[10], q[11]),
+                           e4m3x4(q[12], q[13], q[14], q[15]));
+#pragma unroll
+            for (int i = 0; i < 16; ++i) h[i] = (v[j][i] > 0.0f) ? v[j][i] : 0.0f;             // qu.py:429
+            grid_values16<T, typename SF::POS>(h, sp, delta, q);
+            *reinterpret_cast<uint4*>(blk_p + (kq + 4 * j) * 128 + r * 16) =
+                make_uint4(e4m3x4(q[0], q[1], q[2], q[3]), e4m3x4(q[4], q[5], q[6], q[7]), e4m3x4(q[8], q[9], q[10], q[11]),
+                           e4m3x4(q[12], q[13], q[14], q[15]));
+        }
+        if (kq == 0) {
+            scales[2 * slab * rows_pad + row] = live ? sn : 0.0f;
+            scales[(2 * slab + 1) * rows_pad + row] = live ? sp : 0.0f;
+        }
+    }
+}
+
+// The reference's whole-tensor clip (qu.py:421-422) when the tensor held a NaN: every element becomes NaN, both where() halves 0,
+// every scale 0 and every grid value 0 -- the packing of the all-zero tensor.  workspace = {flag, ticket}: the last CTA leaves it
+// zeroed for the next call.
+__global__ void __launch_bounds__(256) codes_clip_fill_kernel(uint4* __restrict__ codes, size_t n_vec, float* __restrict__ scales,
+                                                              size_t n_scales, unsigned* __restrict__ ws) {
+    if (*reinterpret_cast<volatile unsigned*>(ws) != 0u) {
+        for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n_vec; i += size_t(gridDim.x) * blockDim.x)
+            codes[i] = make_uint4(0u, 0u, 0u, 0u);
+        for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n_scales; i += size_t(gridDim.x) * blockDim.x) scales[i] = 0.0f;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0 && atomicAdd(ws + 1, 1u) == gridDim.x - 1) { ws[0] = 0u; ws[1] = 0u; }
+}
+
+__device__ __forceinline__ void e4m3x16_to_f32(uint4 u, float (&q)[16]) {
+    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+#pragma unroll
+        for (int b = 0; b < 4; b += 2) {
+            const __half2_raw hr = __nv_cvt_fp8x2_to_halfraw2(__nv_fp8x2_storage_t((w[i] >> (8 * b)) & 0xffffu), __NV_E4M3);
+            q[4 * i + b] = __half2float(__ushort_as_half(hr.x));
+            q[4 * i + b + 1] = __half2float(__ushort_as_half(hr.y));
+        }
+    }
+}
+
+// sign-split codes -> values: out[row, c] = T( fl32(qn) * sn + fl32(qp) * sp ), two products and one sum each rounded on its own
+// (qu.py:450; __fmul_rn / __fadd_rn keep ptxas from contracting them into an FMA).  One thread per 16-byte chunk of each half.
+template <typename T>
+__global__ void __launch_bounds__(256) unpack_codes_split_kernel(const uint8_t* __restrict__ codes, const float* __restrict__ scales,
+                                                                 size_t rows, size_t rows_pad, size_t k, T* __restrict__ out) {
+    const size_t groups = k / GK, row_blocks = rows_pad / 8;
+    const size_t n_chunks = groups * row_blocks * 64;
+    for (size_t c = size_t(blockIdx.x) * blockDim.x + threadIdx.x; c < n_chunks; c += size_t(gridDim.x) * blockDim.x) {
+        const size_t blk = c >> 6;
+        const int kc = int(c >> 3) & 7, r = int(c) & 7;
+        const size_t t = blk / row_blocks, rb = blk % row_blocks;
+        const size_t row = rb * 8 + r;
+        if (row >= rows) continue;
+        const uint8_t* pn = codes + (2 * t * row_blocks + rb) * BLK_BYTES + (c & 63) * 16;
+        float qn[16], qp[16];
+        e4m3x16_to_f32(*reinterpret_cast<const uint4*>(pn), qn);
+        e4m3x16_to_f32(*reinterpret_cast<const uint4*>(pn + row_blocks * BLK_BYTES), qp);
+        const float sn = scales[2 * t * rows_pad + row], sp = scales[(2 * t + 1) * rows_pad + row];
+        T* o = out + row * k + t * GK + kc * 16;
+#pragma unroll
+        for (int i = 0; i < 16; ++i) o[i] = T(__fadd_rn(__fmul_rn(qn[i], sn), __fmul_rn(qp[i], sp)));
+    }
+}
+
 // 4-bit storage of the FP4 formats: nibble = sign << 3 | index of |q| in the format's non-negative half grid (ascending);
 // byte i holds elements 2i (low nibble) and 2i + 1 of the codes array, whatever its order.
 struct NibbleLut { uint8_t e4m3[16]; };
@@ -356,7 +481,9 @@ struct GemmCfg {
 // forwards "my stage is full" to the leader; the epilogue warps of both CTAs hand accumulators back to the leader.
 // Measured (profiles/r2_gemm_codes.txt): bit-exact; row scales 2.42 / 2.63 PFLOP/s against 2.36 / 2.52 for single CTAs, groups of 128
 // 1.31 / 1.44 against 1.40 / 1.52 -- so pairs are the default for row scales only.
-template <int TN_, int EC_, int OUT, bool PAIR = false>
+// SPLIT: A is a sign-split operand (depth 2k, pack_codes_split_kernel): A slabs 2t and 2t + 1 both meet B slab t and B's scale set
+// t, so the producer reads B slab i >> 1 for A slab i; the MMA issuer and the epilogue run over the 2k / 128 A slabs unchanged.
+template <int TN_, int EC_, int OUT, bool PAIR = false, bool SPLIT = false>
 __global__ void __launch_bounds__(GemmCfg<TN_, EC_>::THREADS, 1) gemm_codes_kernel(const GemmArgs g) {
     using Cfg = GemmCfg<TN_, EC_>;
     constexpr int TN = Cfg::TN, EC = Cfg::EC;
@@ -422,13 +549,14 @@ __global__ void __launch_bounds__(GemmCfg<TN_, EC_>::THREADS, 1) gemm_codes_kern
                 const size_t b_left = g.n_pad - tn * TN;
                 const uint32_t b_rows = b_left < size_t(TN) ? uint32_t(b_left) : uint32_t(TN);        // last tile column may be half
                 for (uint32_t i = 0; i < slabs; ++i, ++it) {
+                    const uint32_t ib = SPLIT ? i >> 1 : i;                 // B slab of A slab i
                     if (i % gs == 0) {
                         const uint32_t q = gi % Cfg::SC_DEPTH, qn = gi / Cfg::SC_DEPTH;
                         if (qn > 0) mbar_wait(&bar_sempty[q], (qn - 1) & 1);
                         uint8_t* sc = sc0 + size_t(q) * Cfg::SC_BYTES;
                         mbar_arrive_expect_tx(&bar_sfull[q], SA_BYTES + b_rows * 4);
                         bulk_load(sc, g.a_scales + size_t(i / gs) * g.m_pad + tm * TM, SA_BYTES, &bar_sfull[q]);
-                        bulk_load(sc + SA_BYTES, g.b_scales + size_t(i / gs) * g.n_pad + tn * TN, b_rows * 4, &bar_sfull[q]);
+                        bulk_load(sc + SA_BYTES, g.b_scales + size_t(SPLIT ? ib : i / gs) * g.n_pad + tn * TN, b_rows * 4, &bar_sfull[q]);
                         ++gi;
                     }
                     const uint32_t s = it % stages, n = it / stages;
@@ -438,11 +566,11 @@ __global__ void __launch_bounds__(GemmCfg<TN_, EC_>::THREADS, 1) gemm_codes_kern
                         const uint32_t half = b_rows / 2 * GK;             // b_rows is 128 or 256: halves of whole 8-row blocks
                         mbar_arrive_expect_tx(&bar_full[s], A_BYTES + half);
                         bulk_load(st, g.a_codes + (size_t(i) * a_blocks + tm * (TM / 8)) * BLK_BYTES, A_BYTES, &bar_full[s]);
-                        bulk_load(st + A_BYTES, g.b_codes + (size_t(i) * b_blocks + tn * (TN / 8)) * BLK_BYTES + pair_rank * half, half, &bar_full[s]);
+                        bulk_load(st + A_BYTES, g.b_codes + (size_t(ib) * b_blocks + tn * (TN / 8)) * BLK_BYTES + pair_rank * half, half, &bar_full[s]);
                     } else {
                         mbar_arrive_expect_tx(&bar_full[s], A_BYTES + b_rows * GK);
                         bulk_load(st, g.a_codes + (size_t(i) * a_blocks + tm * (TM / 8)) * BLK_BYTES, A_BYTES, &bar_full[s]);
-                        bulk_load(st + A_BYTES, g.b_codes + (size_t(i) * b_blocks + tn * (TN / 8)) * BLK_BYTES, b_rows * GK, &bar_full[s]);
+                        bulk_load(st + A_BYTES, g.b_codes + (size_t(ib) * b_blocks + tn * (TN / 8)) * BLK_BYTES, b_rows * GK, &bar_full[s]);
                     }
                 }
             }
@@ -727,6 +855,74 @@ extern "C" int fpq_unpack_codes(const uint8_t* codes, const float* scales, size_
     return finish_launch();
 }
 
+namespace {
+
+// int_neg_e2m3_pos has no codes form: its negative half grid is the integers 0..32, and 17, 19, ..., 31 are not e4m3 numbers
+int split_codes_format(int split) {
+    if (split < 0 || split >= FPQ_NUM_SPLIT_FORMATS) return FPQ_ERR_ARG;
+    return split == FPQ_SPLIT_INTNEG_E2M3POS ? FPQ_ERR_UNSUPPORTED : FPQ_OK;
+}
+
+template <typename T, bool GELU>
+int launch_pack_split(int split, const T* x, size_t rows, size_t k, unsigned flags, void* workspace, uint8_t* codes, float* scales,
+                      cudaStream_t st) {
+    const size_t rows_pad = fpq_codes_rows_padded(rows);
+    const unsigned grid = grid_for((k / GK) * (rows_pad / 8), 8, 8);
+    unsigned* flag = (flags & FPQ_FLAG_GLOBAL_CLIP) ? static_cast<unsigned*>(workspace) : nullptr;
+    if (split == FPQ_SPLIT_E1M2NEG_E2M1POS)
+        pack_codes_split_kernel<T, FPQ_SPLIT_E1M2NEG_E2M1POS, GELU><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales, flag);
+    else
+        pack_codes_split_kernel<T, FPQ_SPLIT_AFPQ_E2M1, GELU><<<grid, 256, 0, st>>>(x, rows, rows_pad, k, codes, scales, flag);
+    int rc = finish_launch();
+    if (rc != FPQ_OK || flag == nullptr) return rc;
+    const size_t n_vec = 2 * rows_pad * k / 16, n_scales = 2 * (k / GK) * rows_pad;
+    codes_clip_fill_kernel<<<grid_for(n_vec, 256 * 8, 8), 256, 0, st>>>(reinterpret_cast<uint4*>(codes), n_vec, scales, n_scales, flag);
+    return finish_launch();
+}
+
+int pack_split_args(const void* x, size_t rows, size_t k, int split, unsigned flags, const void* workspace, const uint8_t* codes,
+                    const float* scales) {
+    if (k == 0 || k % GK != 0 || k > (SIZE_MAX >> 2)) return FPQ_ERR_ARG;
+    if ((rows && (!x || !codes || !scales)) || !aligned16(x) || !aligned16(codes) || !aligned16(scales)) return FPQ_ERR_ARG;
+    if ((flags & ~FPQ_FLAG_GLOBAL_CLIP) || ((flags & FPQ_FLAG_GLOBAL_CLIP) && !workspace)) return FPQ_ERR_ARG;
+    return split_codes_format(split);
+}
+
+}  // namespace
+
+extern "C" int fpq_pack_codes_signsplit(const void* x, size_t rows, size_t k, int in_dtype, int split_format, unsigned flags, void* workspace,
+                                        uint8_t* codes, float* scales, void* stream) {
+    if (int rc = pack_split_args(x, rows, k, split_format, flags, workspace, codes, scales)) return rc;
+    if (in_dtype != FPQ_F16 && in_dtype != FPQ_F32) return FPQ_ERR_ARG;
+    if (rows == 0) return FPQ_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (in_dtype == FPQ_F16)
+        return launch_pack_split<__half, false>(split_format, static_cast<const __half*>(x), rows, k, flags, workspace, codes, scales, st);
+    return launch_pack_split<float, false>(split_format, static_cast<const float*>(x), rows, k, flags, workspace, codes, scales, st);
+}
+
+extern "C" int fpq_gelu_pack_codes_signsplit(const void* x_f16, size_t rows, size_t k, int split_format, unsigned flags, void* workspace,
+                                             uint8_t* codes, float* scales, void* stream) {
+    if (int rc = pack_split_args(x_f16, rows, k, split_format, flags, workspace, codes, scales)) return rc;
+    if (rows == 0) return FPQ_OK;
+    return launch_pack_split<__half, true>(split_format, static_cast<const __half*>(x_f16), rows, k, flags, workspace, codes, scales,
+                                           static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int fpq_unpack_codes_signsplit(const uint8_t* codes, const float* scales, size_t rows, size_t k, int out_dtype, void* out,
+                                          void* stream) {
+    if (k == 0 || k % GK != 0 || k > (SIZE_MAX >> 2)) return FPQ_ERR_ARG;
+    if ((rows && (!out || !codes || !scales)) || !aligned16(codes)) return FPQ_ERR_ARG;
+    if (out_dtype != FPQ_F16 && out_dtype != FPQ_F32) return FPQ_ERR_ARG;
+    if (rows == 0) return FPQ_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t rows_pad = fpq_codes_rows_padded(rows);
+    const unsigned grid = grid_for(rows_pad * k / 16, 256, 8);
+    if (out_dtype == FPQ_F16) unpack_codes_split_kernel<__half><<<grid, 256, 0, st>>>(codes, scales, rows, rows_pad, k, static_cast<__half*>(out));
+    else unpack_codes_split_kernel<float><<<grid, 256, 0, st>>>(codes, scales, rows, rows_pad, k, static_cast<float*>(out));
+    return finish_launch();
+}
+
 extern "C" int fpq_codes_to_nibbles(const uint8_t* codes, size_t n_codes, int format, uint8_t* nibbles, void* stream) {
     NibbleLut lut;
     if (!half_grid_e4m3(format, lut)) return FPQ_ERR_UNSUPPORTED;
@@ -747,7 +943,7 @@ extern "C" int fpq_nibbles_to_codes(const uint8_t* nibbles, size_t n_codes, int 
 
 namespace {
 
-template <int TN_, int EC_, int OUT>
+template <int TN_, int EC_, int OUT, bool SPLIT>
 int launch_gemm(GemmArgs& g, cudaStream_t st) {
     using Cfg = GemmCfg<TN_, EC_>;
     if (int(g.stages) > Cfg::MAX_STAGES) g.stages = Cfg::MAX_STAGES;
@@ -761,18 +957,18 @@ int launch_gemm(GemmArgs& g, cudaStream_t st) {
     int dev = 0;
     cudaGetDevice(&dev);
     if (!attr_set[dev & 63].load(std::memory_order_acquire)) {
-        if (cudaFuncSetAttribute(gemm_codes_kernel<TN_, EC_, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(Cfg::smem_bytes(Cfg::MAX_STAGES))) != cudaSuccess)
+        if (cudaFuncSetAttribute(gemm_codes_kernel<TN_, EC_, OUT, false, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(Cfg::smem_bytes(Cfg::MAX_STAGES))) != cudaSuccess)
             return finish_launch();
         attr_set[dev & 63].store(true, std::memory_order_release);
     }
     const size_t resident = size_t(sm_count());
     const unsigned grid = unsigned(tiles < resident ? tiles : resident);
-    gemm_codes_kernel<TN_, EC_, OUT><<<grid, Cfg::THREADS, Cfg::smem_bytes(int(g.stages)), st>>>(g);
+    gemm_codes_kernel<TN_, EC_, OUT, false, SPLIT><<<grid, Cfg::THREADS, Cfg::smem_bytes(int(g.stages)), st>>>(g);
     return finish_launch();
 }
 
 // CTA pairs (clusters of two): instantiated for the default tile shape only
-template <int TN_, int EC_, int OUT>
+template <int TN_, int EC_, int OUT, bool SPLIT>
 int launch_gemm_pair(GemmArgs& g, cudaStream_t st) {
     using Cfg = GemmCfg<TN_, EC_>;
     if (g_tun.gemm_stages >= 6 || int(g.stages) > Cfg::MAX_STAGES_PAIR) g.stages = Cfg::MAX_STAGES_PAIR;     // default: as deep as fits
@@ -781,7 +977,7 @@ int launch_gemm_pair(GemmArgs& g, cudaStream_t st) {
     if (tiles_m * tiles_n > 0x7fffffffull) return FPQ_ERR_UNSUPPORTED;
     g.n_tiles = uint32_t(tiles_m * tiles_n);
     g.tiles_n = uint32_t(tiles_n);
-    auto kernel = gemm_codes_kernel<TN_, EC_, OUT, true>;
+    auto kernel = gemm_codes_kernel<TN_, EC_, OUT, true, SPLIT>;
     // per device: resident clusters, 0 = not known yet.  Published after the shared-memory attribute is set, in one atomic, so that
     // a thread that reads a count also sees the attribute (two plain statics could be seen in either order: a grid of 0 clusters)
     static std::atomic<int> max_clusters[64];
@@ -811,18 +1007,18 @@ int launch_gemm_pair(GemmArgs& g, cudaStream_t st) {
     return finish_launch();
 }
 
-template <int OUT>
+template <int OUT, bool SPLIT = false>
 int launch_gemm_tn(GemmArgs& g, cudaStream_t st) {
     const int ec = g_tun.gemm_epi_cols;
     if (g_tun.gemm_tile_n == 128) {
-        if (ec == 32) return launch_gemm<128, 32, OUT>(g, st);
-        if (ec == 64) return launch_gemm<128, 64, OUT>(g, st);
-        return launch_gemm<128, 128, OUT>(g, st);
+        if (ec == 32) return launch_gemm<128, 32, OUT, SPLIT>(g, st);
+        if (ec == 64) return launch_gemm<128, 64, OUT, SPLIT>(g, st);
+        return launch_gemm<128, 128, OUT, SPLIT>(g, st);
     }
-    if (ec == 64) return launch_gemm<256, 64, OUT>(g, st);
+    if (ec == 64) return launch_gemm<256, 64, OUT, SPLIT>(g, st);
     // default (-1): CTA pairs where they were measured faster -- row scales (+3-4 %), not groups of 128 (-6 %)
     const bool pair = g_tun.gemm_pair == 1 || (g_tun.gemm_pair < 0 && g.group_slabs != 1 && g.slabs > 1 && g.m_pad / TM >= 4);
-    return pair ? launch_gemm_pair<256, 128, OUT>(g, st) : launch_gemm<256, 128, OUT>(g, st);
+    return pair ? launch_gemm_pair<256, 128, OUT, SPLIT>(g, st) : launch_gemm<256, 128, OUT, SPLIT>(g, st);
 }
 
 int gemm_common(GemmArgs& g, const uint8_t* a_codes, const float* a_scales, size_t m, const uint8_t* b_codes, const float* b_scales, size_t n,
@@ -863,4 +1059,29 @@ extern "C" int fpq_gemm_codes_sse(const uint8_t* a_codes, const float* a_scales,
     g.row_weight = row_weight;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     return ref_dtype == FPQ_F16 ? launch_gemm_tn<OUT_SSE_F16>(g, st) : launch_gemm_tn<OUT_SSE_F32>(g, st);
+}
+
+extern "C" int fpq_gemm_codes_signsplit(const uint8_t* a_codes, const float* a_scales, size_t m, const uint8_t* b_codes, const float* b_scales,
+                                        size_t n, size_t k, const float* bias, int out_dtype, void* c, size_t ldc, void* stream) {
+    if (m == 0 || n == 0) return FPQ_OK;
+    if (out_dtype != FPQ_F16 && out_dtype != FPQ_F32) return FPQ_ERR_ARG;
+    if (k == 0 || k % GK != 0 || k > (SIZE_MAX >> 2)) return FPQ_ERR_ARG;
+    GemmArgs g;
+    if (int rc = gemm_common(g, a_codes, a_scales, m, b_codes, b_scales, n, 2 * k, GK, bias, c, ldc)) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return out_dtype == FPQ_F16 ? launch_gemm_tn<OUT_F16, true>(g, st) : launch_gemm_tn<OUT_F32, true>(g, st);
+}
+
+extern "C" int fpq_gemm_codes_signsplit_sse(const uint8_t* a_codes, const float* a_scales, size_t m, const uint8_t* b_codes,
+                                            const float* b_scales, size_t n, size_t k, const float* bias, int ref_dtype, const void* ref,
+                                            size_t ldr, const double* row_weight, double* sse, void* stream) {
+    if (m == 0 || n == 0) return FPQ_OK;
+    if ((ref_dtype != FPQ_F16 && ref_dtype != FPQ_F32) || !sse) return FPQ_ERR_ARG;
+    if (k == 0 || k % GK != 0 || k > (SIZE_MAX >> 2)) return FPQ_ERR_ARG;
+    GemmArgs g;
+    if (int rc = gemm_common(g, a_codes, a_scales, m, b_codes, b_scales, n, 2 * k, GK, bias, const_cast<void*>(ref), ldr)) return rc;
+    g.sse = sse;
+    g.row_weight = row_weight;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return ref_dtype == FPQ_F16 ? launch_gemm_tn<OUT_SSE_F16, true>(g, st) : launch_gemm_tn<OUT_SSE_F32, true>(g, st);
 }

@@ -142,7 +142,9 @@ def search_layer_lowbit(weight: torch.Tensor, activations: Sequence[torch.Tensor
     """The loss table of `search_layer_batched` with the quantized layer evaluated from codes on the tensor cores and compared
     with y_fp inside the GEMM's epilogue (lowbit.linear_codes_sse: SURVEY.md section 8 f3): every candidate pair costs one
     low-bit GEMM that writes nothing, every activation format one quantizer pass, every weight format one; the only library
-    GEMM left is y_fp.  Symmetric formats only.  Rounding is the kernel tie rule of the evaluation path
+    GEMM left is y_fp.  Weight formats are symmetric; activation formats may also be the sign-split formats with a codes form
+    (lowbit.SPLIT_FORMATS, per="group": the fc2 search), packed without the whole-tensor clip as `quantize` applies none.
+    Rounding is the kernel tie rule of the evaluation path
     (fp_quant_*_per_group_cuda) where the search scripts' FPQuant uses torch.argmin (search_fp4_format.py:340-363): the two
     differ on exact midpoints only.  The products are exact where the reference's fp16 / fp32 GEMMs round; measured agreement
     of the loss tables: tests/test_gpu_gemm_codes.py."""
@@ -162,7 +164,7 @@ def search_layer_lowbit(weight: torch.Tensor, activations: Sequence[torch.Tensor
         ws = row_w[r0:r0 + max_rows].contiguous()
         y_fp = torch.matmul(xs, weight.T.to(xs.dtype)).contiguous()
         for ai, af in enumerate(act_formats):
-            a = lowbit.pack_codes(xs, af, per_row)
+            a = lowbit.pack_codes(xs, af, per_row, global_clip=False)
             for wi in range(len(weight_formats)):
                 lowbit.linear_codes_sse(a, wq[wi], y_fp, None, loss[wi, ai:ai + 1], ws)
     return loss

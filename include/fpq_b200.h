@@ -354,6 +354,49 @@ FPQ_API int fpq_gemm_codes_sse(const uint8_t *a_codes, const float *a_scales, si
                    const float *b_scales, size_t n, size_t k, size_t scale_group, const float *bias, int ref_dtype,
                    const void *ref, size_t ldr, const double *row_weight, double *sse, void *stream);
 
+/* ------------------------------------------------------------------------------------------------------------------
+ * Sign-split operands (the fc2 input, fp_quant_e1m2_neg_e2m1_pos_per_group_cuda qu.py:415-452, fp4_afpq_per_group_cuda
+ * qu0.py:498-535).  Each 128-group t of a row has two scales, sn for x <= 0 and sp for x > 0, and stands for qn*sn + qp*sp, one of
+ * qn, qp being 0 in every element.  It is stored as an operand of depth 2k in the layout above, with its slabs interleaved:
+ *   codes  : 2 * rows_pad * k bytes; slab 2t = the negative half's grid values of group t (0 where x > 0),
+ *                                    slab 2t+1 = the positive half's (0 where x <= 0)
+ *   scales : fp32 [2k/128][rows_pad]; row 2t = sn, row 2t+1 = sp; 0 for the padding rows
+ * Formats: FPQ_SPLIT_E1M2NEG_E2M1POS (e1m2 / e2m1 halves) and FPQ_SPLIT_AFPQ_E2M1 (mirrored e2m1 / e2m1), both subsets of e4m3.
+ * FPQ_SPLIT_INTNEG_E2M3POS is refused with FPQ_ERR_UNSUPPORTED: its negative half grid is the integers 0..32, and 17, 19, ..., 31
+ * are not e4m3 numbers.  Every pairing of a split half with a symmetric weight format lies inside the exact-accumulation
+ * envelope (the widest, e2m1 x e3m2: 128 * 12 * 448 ~ 2^19.4), so the split GEMM is bit-exact against the oracle.
+ * ------------------------------------------------------------------------------------------------------------------ */
+/*
+ * x: [rows, k] contiguous, FPQ_F16 | FPQ_F32, 16-byte aligned, k % 128 == 0; kernel tie rule.  Numerics contract:
+ * fpq_unpack_codes_signsplit of the result is bit-identical to fpq_fake_quant_signsplit(x, rows * k / 128, 128, in_dtype, in_dtype,
+ * split_format, FPQ_TIE_KERNEL, flags); the scales of an fp16 input are the fp16-rounded sn / sp stored as fp32.
+ * flags: 0 or FPQ_FLAG_GLOBAL_CLIP with the {flag, ticket} workspace of fpq_fake_quant_signsplit: if the tensor holds a NaN, the
+ * result is the packing of the all-zero tensor (every code and every scale 0), which is what the reference's clip produces (every
+ * element +0); the last CTA zeroes the workspace again.  Without the flag a NaN element counts as 0 locally (qu.py:428-429).
+ */
+FPQ_API int fpq_pack_codes_signsplit(const void *x, size_t rows, size_t k, int in_dtype, int split_format, unsigned flags,
+                   void *workspace, uint8_t *codes, float *scales, void *stream);
+/* The fc2 input straight from the fp16 fc1 output in one pass: fpq_pack_codes_signsplit(gelu_tanh(x_f16)), GELU as in
+ * fpq_gelu_fake_quant_signsplit (fp16-rounded before quantization).  Arguments and contract as fpq_pack_codes_signsplit. */
+FPQ_API int fpq_gelu_pack_codes_signsplit(const void *x_f16, size_t rows, size_t k, int split_format, unsigned flags,
+                   void *workspace, uint8_t *codes, float *scales, void *stream);
+/* out[r, c] = out_dtype( fl32(qn) * sn + fl32(qp) * sp ), both products and the sum each rounded on its own (qu.py:450). */
+FPQ_API int fpq_unpack_codes_signsplit(const uint8_t *codes, const float *scales, size_t rows, size_t k, int out_dtype,
+                   void *out, void *stream);
+/*
+ * F.linear(A, W, bias) for a sign-split A ([m, k], depth-2k codes) and a W = [n, k] scaled per 128-group (fpq_pack_codes with
+ * scale_group = 128): A slabs 2t and 2t+1 both meet W slab t with W's scale of group t, so
+ *   C[i, j] = bias[j] + fma-chain over the 2k/128 A slabs u (ascending) of  (P_u[i, j] * sa[u, i]) * sw[u >> 1, j]
+ * which is, by construction, fpq_gemm_codes / oracle/gemm_codes.c on A' = the [m, 2k] operand and W' = W with every 128-slab
+ * (and its scale) repeated twice.  Output, bias, alignment, tunables and the SSE form: as fpq_gemm_codes / fpq_gemm_codes_sse.
+ */
+FPQ_API int fpq_gemm_codes_signsplit(const uint8_t *a_codes, const float *a_scales, size_t m, const uint8_t *b_codes,
+                   const float *b_scales, size_t n, size_t k, const float *bias, int out_dtype, void *c, size_t ldc,
+                   void *stream);
+FPQ_API int fpq_gemm_codes_signsplit_sse(const uint8_t *a_codes, const float *a_scales, size_t m, const uint8_t *b_codes,
+                   const float *b_scales, size_t n, size_t k, const float *bias, int ref_dtype, const void *ref, size_t ldr,
+                   const double *row_weight, double *sse, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
